@@ -15,7 +15,7 @@ same number of postings and gathers the same number of chunk rows per step as th
 all-gather, 4-word all-reduce of the min-max bounds, local top-100 records to the owner) runs as NCCL calls enqueued on
 the compute stream inside the library.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `value` = hybrid queries/s with the inputs resident in HBM (CUDA events, max over
 ranks); `e2e` = the same through the C ABI with PINNED HOST buffers (H2D of query CSR + query vectors and D2H of the
@@ -51,6 +51,7 @@ MAX_OUT = 100
 SEED = 1234
 METRIC = "hybrid_queries_per_sec"
 UNIT = "queries/s"
+DUMP_BYTES = 64 << 20
 
 
 def workload_name(n_docs, n_chunks, batch):
@@ -549,11 +550,28 @@ def dense_c4_supplement(corpus_rank, world, dev, local_rank, id_bytes, peak, top
                                "against fp32 dot products of the stored rows, tolerance 2e-3 relative"}}
 
 
+def dump_outputs(path, out):
+    """Writes what one hybrid call returned (`out_*` of `mse_hybrid_search_batch`: doc, score, orig, chunk, count, rows)
+    as <path>/hybrid_<name>.npy: scores as float32; ids, chunk rows and counts as float64 (exact below 2**53).  Above
+    DUMP_BYTES in all, a fixed seeded sample of the queries is written, their batch indices in hybrid_query_index.npy."""
+    names = ("doc", "score", "orig", "chunk", "count", "rows")
+    arrays = {n: x.cpu().numpy().astype(np.float32 if x.is_floating_point() else np.float64) for n, x in zip(names, out)}
+    n_q = arrays["count"].shape[0]
+    per_query = sum(a[:1].nbytes for a in arrays.values())
+    if per_query * n_q > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(SEED).choice(n_q, DUMP_BYTES // (per_query + 8), replace=False))
+        arrays = {n: a[keep] for n, a in arrays.items()}
+        arrays["query_index"] = keep.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for n, a in arrays.items():
+        np.save(os.path.join(path, f"hybrid_{n}.npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps (batches) of the headline value and e2e legs")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--docs", type=int, default=N_DOCS, help="experiments only: a smaller corpus (the line then says so)")
@@ -569,7 +587,14 @@ def main():
     ap.add_argument("--neg-lookup", type=int, default=1)
     ap.add_argument("--range-docs", type=int, default=0)
     ap.add_argument("--no-class-term", action="store_true", help="experiments: leave the posting class bits on the default term")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed hybrid step returned as DIR/hybrid_*.npy (N > 1: rank 0's block); the "
+                         "inputs depend only on the arguments, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -683,7 +708,8 @@ def main():
     stats = nat.bm25_stats()                             # counters of the last step
     status_total = status_acc.cpu().tolist()
     rows_per_query = float(out[5].float().mean().item())
-    gpu_doc, gpu_score, gpu_count = (x.cpu().numpy() for x in (out[0], out[1], out[4]))     # last step (not the parity batch)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)             # before the parity leg reuses `out`
 
     note(f"value leg done: {value:.0f} {UNIT}")
     # ---- e2e: pinned host buffers through the C ABI, two streams alternating ---------------------------------

@@ -7,6 +7,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import shutil
 import subprocess
 import sys
 from typing import Optional, Tuple
@@ -41,7 +42,8 @@ def build(verbose: bool = False) -> str:
     deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cu", ".cuh"))] + [HEADER]
     if os.path.exists(LIB_PATH) and all(os.path.getmtime(LIB_PATH) >= os.path.getmtime(d) for d in deps):
         return LIB_PATH
-    nvcc = os.environ.get("NVCC", "nvcc")
+    nvcc = os.environ.get("NVCC") or shutil.which("nvcc") or \
+        os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "nvcc")      # a shell without the toolkit on PATH
     extra = os.environ.get("MSE_NVCC_FLAGS", "").split()          # experiments, e.g. -DMSE_BM25_RANGE16=4096
     cmd = [nvcc] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-o", LIB_PATH, src]
     r = subprocess.run(cmd, capture_output=True, text=True)
@@ -201,6 +203,7 @@ class NativeIndex:
         if getattr(self, "_h", None) is not None and self._h.value:
             lib().mse_index_destroy(self._h)
             self._h = C.c_void_p()
+        self._borrowed = None                            # a closed index no longer reads the tensor lent by dense_load
 
     def __del__(self):
         try:
