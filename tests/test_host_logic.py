@@ -7,6 +7,7 @@ import sqlite3
 
 import numpy as np
 import pytest
+import torch
 
 import mse_b200
 import mse_testlib as helpers
@@ -544,3 +545,44 @@ def test_hosted_reference_timing_record():
     assert 0 < rec["hosted_reference"]["queries_per_s"] < rec["oracle_port"]["faithful_queries_per_s"] < rec["oracle_port"]["fast_queries_per_s"]
     cited = bench.hosted_reference_c1()
     assert cited is not None and cited["queries_per_s"] == rec["hosted_reference"]["queries_per_s"] and "not by this run" in cited["source"]
+
+
+def test_exact_dense_rule_rejects_simulated_kernel_defects():
+    """The rule of tests/test_gpu_dense_exact.py (mse_testlib.assert_dense_exact against the exact-input reference) passes
+    a correct fp32-accumulate scan and fails two defects the 2e-3 rule lets through: the fp32-query GEMV rounding its
+    query to bf16, and the tensor-core scan accumulating in fp16 (a wrong D format in the instruction descriptor) — also
+    at 1e-4, the widest the dense tests may use."""
+    d = synthetic.make_dense_corpus(2000, seed=5, device="cpu", dtype=torch.float32)
+    off = d.doc_chunk_off.numpy()
+    stored = helpers.bf16_round(d.emb.numpy())
+    Q = synthetic.make_query_vectors(24, seed=108, normalize=True)
+    top_k = 100
+    ref32 = helpers.dense_exact_reference(stored, off, Q, False, top_k)
+    ref16 = helpers.dense_exact_reference(stored, off, Q, True, top_k)
+    has = np.flatnonzero(off[1:] > off[:-1])
+
+    def scan(row_scores):
+        best = np.maximum.reduceat(row_scores, off[has])
+        o = np.argsort(-best.astype(np.float64), kind="stable")[:top_k]
+        return has[o], best[o].astype(np.float32), len(o)
+
+    def fp16_accumulate(q):
+        acc = np.zeros(len(stored), np.float16)
+        for k0 in range(0, 768, 16):                                   # one K = 16 MMA step at a time
+            acc = (acc.astype(np.float32) + stored[:, k0:k0 + 16] @ q[k0:k0 + 16]).astype(np.float16)
+        return acc.astype(np.float32)
+
+    def passes(row_scores, ref, i, rtol):
+        try:
+            helpers.assert_dense_exact(*scan(row_scores), ref, i, rtol=rtol)
+            return True
+        except AssertionError:
+            return False
+
+    for i, q in enumerate(Q):
+        qb = helpers.bf16_round(q)
+        assert passes(stored @ q, ref32, i, helpers.DENSE_EXACT_RTOL)                  # K3: fp32 query, fp32 sums
+        assert passes(stored @ qb, ref16, i, helpers.DENSE_EXACT_RTOL)                 # K4: bf16 query, fp32 sums
+        for rtol in (helpers.DENSE_EXACT_RTOL, 1e-4):
+            assert not passes(stored.astype(np.float64) @ qb.astype(np.float64), ref32, i, rtol)
+            assert not passes(fp16_accumulate(qb), ref16, i, rtol)
