@@ -45,7 +45,7 @@ struct mse_index {
 
     bool has_bm25 = false;
     Bm25Dev bm{};
-    DevBuf term_off, post2, skip, skip_row, imp_levels, idf, neg_row, neg_imp;
+    DevBuf term_off, post2, skip, skip_row, imp_levels, imp_pair, idf, neg_row, neg_imp;
     std::vector<int64_t> h_term_off;
     std::vector<int32_t> h_neg_row;      // term -> dense row (-1: none), host copy
     int64_t neg_stride = 0;
@@ -543,6 +543,21 @@ int mse_index_destroy(mse_index* ix) {
     return MSE_OK;
 }
 
+// Paired impact table of the class term `cls_term` (dense row `row`, its class bits already in the postings): see
+// bm25_paired_levels_kernel.  Needs term_off, post2, idf and neg_imp in place.
+static int build_paired_levels(mse_index* ix, int64_t n_terms, int32_t cls_term, int32_t row, cudaStream_t st) {
+    int rc;
+    if ((rc = ix->imp_pair.ensure(sizeof(float) * kImpLevels * size_t(std::max<int64_t>(n_terms, 1))))) return rc;
+    if (n_terms > 0) {
+        bm25_paired_levels_kernel<<<unsigned(n_terms), kImpThreads, 0, st>>>(ix->term_off.as<int64_t>(), ix->post2.as<int2>(),
+                                                                            ix->idf.as<float>(), ix->neg_imp.as<float>() + int64_t(row) * ix->neg_stride,
+                                                                            cls_term, ix->imp_pair.as<float>(), n_terms);
+        MSE_CUDA_TRY(cudaGetLastError());
+    }
+    MSE_CUDA_TRY(cudaStreamSynchronize(st));
+    return MSE_OK;
+}
+
 int mse_index_set_option(mse_index* ix, const char* name, int64_t value) {
     if (!ix || !name) { set_error("null argument"); return MSE_ERR_INVALID; }
     std::lock_guard<std::mutex> lk(ix->mu);
@@ -568,8 +583,16 @@ int mse_index_set_option(mse_index* ix, const char* name, int64_t value) {
             MSE_CUDA_TRY(cudaDeviceSynchronize());
         }
         ix->bm.cls_row = row;
+        ix->bm.imp_pair = nullptr;                           // the paired table belongs to the class term: rebuild it
+        int rc;
+        if ((rc = build_paired_levels(ix, ix->bm.n_terms, int32_t(value), row, 0))) return rc;
+        ix->bm.imp_pair = ix->opt_tau_init ? ix->imp_pair.as<float>() : nullptr;
     }
-    else if (!strcmp(name, "bm25_tau_init")) { ix->opt_tau_init = value; ix->bm.imp_levels = (value && ix->has_bm25) ? ix->imp_levels.as<float>() : nullptr; }
+    else if (!strcmp(name, "bm25_tau_init")) {
+        ix->opt_tau_init = value;
+        ix->bm.imp_levels = (value && ix->has_bm25) ? ix->imp_levels.as<float>() : nullptr;
+        ix->bm.imp_pair = (value && ix->has_bm25 && ix->bm.cls_row >= 0) ? ix->imp_pair.as<float>() : nullptr;
+    }
     else if (!strcmp(name, "bm25_queries_per_item")) ix->opt_qpi = value;
     else if (!strcmp(name, "bm25_cand_cap")) ix->opt_cand_cap = value;
     else if (!strcmp(name, "bm25_use_tau")) ix->opt_use_tau = value;
@@ -715,7 +738,7 @@ int mse_bm25_load(mse_index* ix, int64_t n_terms, int64_t n_docs, int64_t doc_ba
         }
     }
     {   // dense impact rows of the negative-idf terms (df > N/2), largest first, within a memory budget
-        ix->bm.neg_row = nullptr; ix->bm.neg_imp = nullptr; ix->bm.neg_stride = 0; ix->bm.cls_row = -1;
+        ix->bm.neg_row = nullptr; ix->bm.neg_imp = nullptr; ix->bm.neg_stride = 0; ix->bm.cls_row = -1; ix->bm.imp_pair = nullptr;
         std::vector<std::pair<int64_t, int32_t>> neg;          // (df, term)
         for (int64_t t = 0; t < n_terms; ++t)
             if (h_idf[t] < 0.f && ix->h_term_off[t + 1] > ix->h_term_off[t]) neg.emplace_back(ix->h_term_off[t + 1] - ix->h_term_off[t], int32_t(t));
@@ -749,6 +772,7 @@ int mse_bm25_load(mse_index* ix, int64_t n_terms, int64_t n_docs, int64_t doc_ba
                 MSE_CUDA_TRY(cudaGetLastError());
                 MSE_CUDA_TRY(cudaStreamSynchronize(st));
                 ix->bm.cls_row = 0;
+                if ((rc = build_paired_levels(ix, n_terms, h_row_term[0], 0, st))) return rc;
             }
         } else {
             ix->neg_row.release(); ix->neg_imp.release();
@@ -760,6 +784,7 @@ int mse_bm25_load(mse_index* ix, int64_t n_terms, int64_t n_docs, int64_t doc_ba
     ix->bm.post2 = ix->post2.as<int2>();
     ix->bm.idf = ix->idf.as<float>();
     ix->bm.imp_levels = (ix->opt_tau_init && n_terms > 0 && n_docs > 0) ? ix->imp_levels.as<float>() : nullptr;
+    ix->bm.imp_pair = (ix->opt_tau_init && ix->bm.cls_row >= 0) ? ix->imp_pair.as<float>() : nullptr;
     ix->bm.n_terms = n_terms; ix->bm.n_docs = n_docs; ix->bm.n_postings = P;
     ix->bm.doc_base = uint32_t(doc_base); ix->bm.k1 = k1;
     ix->has_bm25 = true;

@@ -63,6 +63,8 @@ struct Bm25Dev {                                 // device-resident index of one
     const int64_t* skip_row;     //   first posting with doc >= g * skip_docs, g = 0..n_skip; skip_row[t] = first entry of term t, -1 = none
     int32_t skip_docs, n_skip;   //   granularity in docs (0 = no table) and ceil(n_docs / skip_docs)
     const float* imp_levels;     // [n_terms * kImpLevels] lower bound of the (64 << l)-th largest tf/(tf+norm) of a term, 0 = unknown
+    const float* imp_pair;       // [n_terms * kImpLevels] the same for idf_t * imp_t(d) + idf_a * imp_a(d) over the postings of t, a =
+                                 //   the class term (cls_row); -inf = unknown (idf_t <= 0, t == a, or too few postings)
     const int32_t* neg_row;      // [n_terms] row of the term in neg_imp, -1 = none.  Terms with idf < 0 (df > N/2) get a DENSE
     const float* neg_imp;        //   impact row neg_imp[row * neg_stride + doc] (0 where the doc lacks the term): with
     int64_t neg_stride;          //   min_score >= 0 their postings are never streamed, see bm25_score_kernel
@@ -126,14 +128,23 @@ __device__ __forceinline__ int64_t lower_bound_doc(const int2* __restrict__ pd, 
 // alone is >= w_t * imp_r(t); the other terms of the query add at least the (negative) sum of the negative
 // weights (0 < tf/(tf+norm) < 1).  So r >= top_k candidates score >= max_t w_t * imp_r(t) + sum of negative
 // weights, and nothing below that value can reach the top-k.  (The bound only filters candidates; results stay exact.)
+// Charging the class term a (the always-term, in ~95 % of the documents) its full weight wastes most of the bound: its
+// mean impact is well below 1 and it is 0 where a document lacks the term.  When the query's looked-up class slot has
+// qtf 1, the paired table charges it per document instead: r postings d of a term t with idf_t > 0 have
+// idf_t * imp_t(d) + idf_a * imp_a(d) >= L_t(r), so their score is >= (k1+1) * L_t(r) + the OTHER negative weights
+// (qtf_t >= 1 only adds to the t part).  The larger of the two bounds is used.
+// Slack: with at most 32 + 1 round-down FMAs over contributions of magnitude <= mag, the score kernels' fp32 score is
+// within 33 * 2^-23 * mag < 4e-6 * mag of the exact one; the weights and the bound's own arithmetic round to nearest.
 // Also sets maxbin[q], the top histogram bin the bound refresh starts from, to the bin of the query's score ceiling
 // (sum of the positive weights), so that the score kernel needs no atomicMax per candidate.
 __device__ __forceinline__ uint32_t bm25_initial_bound(const Bm25Dev& ix, const Bm25Work& w, int q) {
     int lv = 0;
     while (lv < 7 && (64 << lv) < w.ts.top_k) ++lv;
     const bool have_level = ix.imp_levels != nullptr && (64 << lv) >= w.ts.top_k;
+    const bool have_pair = have_level && ix.imp_pair != nullptr && w.neg_lookup && ix.cls_row >= 0;
     const int64_t need = int64_t(64) << lv;
     float best = 0.f, neg = 0.f, mag = 0.f, pos = 0.f, wq = 0.f;
+    float pbest = -INFINITY, cls_w = 0.f, neg_rest = 0.f;      // paired bound: best L_t(r), class slot weight, other negative weights
     uint32_t look_n = 0u, look_w = 0u, look_row = 0u, neg_streamed = 0u;
     for (int s = w.q_off[q]; s < w.q_off[q + 1]; ++s) {
         const int t = w.q_term[s];
@@ -147,19 +158,29 @@ __device__ __forceinline__ uint32_t bm25_initial_bound(const Bm25Dev& ix, const 
         } else if (wt < 0.f) {
             neg_streamed = 0x100u;
         }
-        if (w.neg_lookup && wt < 0.f && ix.cls_row >= 0 && ix.neg_row[t] == ix.cls_row) wq = -wt * 0.0625f;   // (distinct terms: at most one such slot)
+        const bool cls = w.neg_lookup && wt < 0.f && ix.cls_row >= 0 && ix.neg_row[t] == ix.cls_row;
+        if (cls) wq = -wt * 0.0625f;                                  // (distinct terms: at most one such slot)
         mag += fabsf(wt);
-        if (wt < 0.f) neg += wt;
-        else {
+        if (wt < 0.f) {
+            neg += wt;
+            if (cls && w.q_tf[s] == 1 && cls_w == 0.f) cls_w = wt; else neg_rest += wt;
+        } else {
             pos += wt;
-            if (have_level && df >= need) best = fmaxf(best, wt * ix.imp_levels[int64_t(t) * kImpLevels + lv]);
+            if (have_level && df >= need) {
+                best = fmaxf(best, wt * ix.imp_levels[int64_t(t) * kImpLevels + lv]);
+                if (have_pair && ix.idf[t] > 0.f) pbest = fmaxf(pbest, ix.imp_pair[int64_t(t) * kImpLevels + lv]);
+            }
         }
     }
     w.ts.maxbin[q] = float_to_key(pos * 1.001f + 1e-30f) >> kHistShift;
     w.cls_wq[q] = wq;
     w.inv_unit[q] = pos > 0.f ? 60000.0f / pos : 0.f;
     w.qinfo[q] = make_uint4(look_n | neg_streamed, look_w, look_row, __float_as_uint(wq));
-    const float bound = best * (1.0f - 1e-5f) + neg - 4e-6f * mag;     // slack for the fp32 summation of the score kernel
+    float bound = best * (1.0f - 1e-5f) + neg - 4e-6f * mag;           // slack for the fp32 summation of the score kernel
+    if (cls_w < 0.f && pbest > -INFINITY) {
+        const float pb = (ix.k1 + 1.0f) * pbest;                        // (may be negative)
+        bound = fmaxf(bound, pb - 1e-5f * fabsf(pb) + neg_rest - 4e-6f * mag);
+    }
     if (!w.use_tau || !(bound > 0.f)) return w.min_key;
     const uint32_t key = float_to_key(bound);
     return key > w.min_key ? key : w.min_key;
@@ -669,32 +690,17 @@ bm25_skip_build_kernel(const int64_t* __restrict__ term_off, const int2* __restr
         row[g] = (g == n_skip) ? uint32_t(e - a) : uint32_t(lower_bound_doc(post2, a, e, int64_t(g) * skip_docs) - a);
 }
 
-// Per-term impact table (load time): for l = 0..6 a LOWER bound of the (64 << l)-th largest tf/(tf+norm) among the
-// postings of the term, found with a two-level 256-bin histogram of the 16-bit fixed-point impact; 0 when the
-// term has fewer postings.  One CTA per term.
+// Rank levels of a term's postings [a, e) under a 16-bit code (one CTA, kImpThreads threads, df = e - a >= 64): for
+// l = 0..6 the code of the (64 << l)-th largest posting, -1 when the term has fewer postings, found with a two-level
+// 256-bin histogram.  Returns the codes in the shared array s_low (read by the calling CTA after this returns).
 constexpr int kImpThreads = 256;
-__global__ void __launch_bounds__(kImpThreads)
-bm25_impact_levels_kernel(const int64_t* __restrict__ term_off, const int32_t* __restrict__ post_doc,
-                          const int32_t* __restrict__ post_tf, const float* __restrict__ doc_norm,
-                          float* __restrict__ imp_levels, int64_t n_terms) {
+template <class Code>
+__device__ __forceinline__ const int* bm25_rank_codes(int64_t a, int64_t e, Code fixed16) {
     __shared__ int h1[256];
     __shared__ int h2[7][256];
     __shared__ int s_bin[7], s_above[7], s_low[7];
-    const int64_t t = blockIdx.x;
-    if (t >= n_terms) return;
     const int tid = threadIdx.x;
-    const int64_t a = term_off[t], e = term_off[t + 1];
     const int64_t df = e - a;
-    if (df < 64) {
-        if (tid < kImpLevels) imp_levels[t * kImpLevels + tid] = 0.f;
-        return;
-    }
-    auto fixed16 = [&](int64_t i) {
-        const float tf = float(post_tf[i]);
-        const float imp = tf / (tf + doc_norm[post_doc[i]]);
-        const int u = int(imp * 65536.0f);
-        return u < 0 ? 0 : (u > 65535 ? 65535 : u);
-    };
     h1[tid] = 0;
     for (int l = 0; l < 7; ++l) h2[l][tid] = 0;
     if (tid < 7) { s_bin[tid] = -1; s_above[tid] = 0; s_low[tid] = -1; }
@@ -721,15 +727,69 @@ bm25_impact_levels_kernel(const int64_t* __restrict__ term_off, const int32_t* _
         const int r = (64 << tid) - s_above[tid];
         int run = 0;
         for (int b = 255; b >= 0; --b) {
-            if (run + h2[tid][b] >= r) { s_low[tid] = b; break; }
+            if (run + h2[tid][b] >= r) { s_low[tid] = (s_bin[tid] << 8) | b; break; }
             run += h2[tid][b];
         }
     }
     __syncthreads();
+    return s_low;
+}
+
+// Per-term impact table (load time): for l = 0..6 a LOWER bound of the (64 << l)-th largest tf/(tf+norm) among the
+// postings of the term, the 16-bit fixed-point impact rounded down; 0 when the term has fewer postings.  One CTA per term.
+// (The minimum of 4 CTAs per SM leaves ptxas 64 registers: left alone it picks 32 and spills.)
+__global__ void __launch_bounds__(kImpThreads, 4)
+bm25_impact_levels_kernel(const int64_t* __restrict__ term_off, const int32_t* __restrict__ post_doc,
+                          const int32_t* __restrict__ post_tf, const float* __restrict__ doc_norm,
+                          float* __restrict__ imp_levels, int64_t n_terms) {
+    const int64_t t = blockIdx.x;
+    if (t >= n_terms) return;
+    const int tid = threadIdx.x;
+    const int64_t a = term_off[t], e = term_off[t + 1];
+    if (e - a < 64) {
+        if (tid < kImpLevels) imp_levels[t * kImpLevels + tid] = 0.f;
+        return;
+    }
+    const int* code = bm25_rank_codes(a, e, [=](int64_t i) {
+        const float tf = float(post_tf[i]);
+        const float imp = tf / (tf + doc_norm[post_doc[i]]);
+        const int u = int(imp * 65536.0f);
+        return u < 0 ? 0 : (u > 65535 ? 65535 : u);
+    });
+    if (tid < kImpLevels) imp_levels[t * kImpLevels + tid] = (tid < 7 && code[tid] >= 0) ? float(code[tid]) / 65536.0f : 0.f;
+}
+
+// Paired impact table (load time, rebuilt whenever the class row changes): for every term t with idf_t > 0 other than
+// the class term a, and l = 0..6, a LOWER bound L_t(64 << l) of the (64 << l)-th largest
+//     v(d) = idf_t * imp_t(d) + idf_a * imp_a(d)        (idf_a < 0; imp_a(d) = 0 where d lacks a)
+// over the postings d of t, from the fp32 impacts the score kernels use (postings, dense class row).  v lies in
+// [idf_a, idf_t]; it is formed in double without contraction (tests/bm25_seed_checker.py::paired_levels restates it
+// operation by operation), coded as floor(65536 * (v - idf_a) / (idf_t - idf_a)) and decoded 2^-30 of the range lower (far
+// beyond the double rounding of the code), rounded down to fp32.  -inf where there is no bound.  One CTA per term.
+__global__ void __launch_bounds__(kImpThreads)
+bm25_paired_levels_kernel(const int64_t* __restrict__ term_off, const int2* __restrict__ post2, const float* __restrict__ idf,
+                          const float* __restrict__ cls_imp, int32_t cls_term, float* __restrict__ imp_pair, int64_t n_terms) {
+    const int64_t t = blockIdx.x;
+    if (t >= n_terms) return;
+    const int tid = threadIdx.x;
+    const int64_t a = term_off[t], e = term_off[t + 1];
+    const double it = double(idf[t]), ia = double(idf[cls_term]);
+    if (e - a < 64 || !(it > 0.0) || !(ia < 0.0) || t == cls_term) {
+        if (tid < kImpLevels) imp_pair[t * kImpLevels + tid] = -INFINITY;
+        return;
+    }
+    const double range = it - ia, scale = 65536.0 / range;
+    const int* code = bm25_rank_codes(a, e, [=](int64_t i) {
+        const int2 p = post2[i];
+        const double v = __dadd_rn(__dmul_rn(it, double(__int_as_float(p.y))), __dmul_rn(ia, double(cls_imp[uint32_t(p.x) & kDocMask])));
+        const double u = floor(__dmul_rn(__dsub_rn(v, ia), scale));
+        return u < 0.0 ? 0 : (u > 65535.0 ? 65535 : int(u));
+    });
     if (tid < kImpLevels) {
-        float v = 0.f;
-        if (tid < 7 && s_bin[tid] >= 0 && s_low[tid] >= 0) v = float((s_bin[tid] << 8) | s_low[tid]) / 65536.0f;
-        imp_levels[t * kImpLevels + tid] = v;
+        float v = -INFINITY;
+        if (tid < 7 && code[tid] >= 0)
+            v = __double2float_rd(__dsub_rn(__dadd_rn(ia, __dmul_rn(double(code[tid]), range / 65536.0)), range * 0x1p-30));
+        imp_pair[t * kImpLevels + tid] = v;
     }
 }
 
