@@ -120,6 +120,8 @@ int mse_index_destroy(mse_index* idx);
  *   "dense_gemm_min_batch"   smallest batch routed to the tcgen05 GEMM kernel (default 8; faster from 3 on, but queries are rounded to bf16 there)
  *   "dense_gemm_pair_mode"   batches of 129..256 queries run as clusters of two CTAs: 1 (default) = every E tile TMA-multicast into
  *                            both CTAs, cta_group::1 MMAs; 2 = cta_group::2 MMAs issued by the leader CTA, E stages split
+ *   "rerank_mode"            rerank of batches the small-batch split does not take: 1 (default) = prep, unit scan, persistent
+ *                            gather and fuse kernels; 0 = one CTA per query (rerank_kernel).  Identical results
  *   "timers"                 1 (default) = bracket the kernels with CUDA events (mse_kernel_time), 0 = off
  *   "reset_timers"           any value: zero the accumulated kernel timers
  * Environment: MSE_DEBUG_SYNC=1 synchronises after every BM25 kernel so that a device fault names its kernel. */

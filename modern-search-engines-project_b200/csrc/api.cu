@@ -20,6 +20,7 @@
 #include "hybrid_shard.cuh"
 #include "rerank.cuh"
 #include "rerank_shard.cuh"
+#include "rerank_split.cuh"
 #include "topk.cuh"
 #include "workspace.cuh"
 
@@ -69,6 +70,8 @@ struct mse_index {
     int64_t stats[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     std::atomic<int> u16_backoff{0};              // calls the fp32 score kernel still serves after a hostile batch (bm25_enqueue)
     int score_ctas_per_sm[3] = {0, 0, 0};         // occupancy of the score kernel (fp32 scan / fp32 hit read-out / two-phase) at its default range
+    int64_t opt_rerank_mode = 1;                  // batches past the small-batch split: 0 = rerank_kernel, 1 = prep / gather / fuse kernels
+    int gather_ctas_per_sm = 0;                   // occupancy of rerank_gather_kernel (its persistent grid)
 };
 
 namespace {
@@ -416,17 +419,21 @@ int rerank_enqueue(mse_index* ix, Lease& L, int32_t B, RerankArgs a) {
     int rc;
     if (!a.url_group && ix->n_url_groups >= ix->dn.n_docs && ix->dn.doc_base == 0 && ix->n_url_groups > 0) a.url_group = ix->url_group.as<int32_t>();
     const int slices = (B * 4 <= ix->sm_count && ix->dn.doc_base == 0) ? std::min(32, std::max(1, ix->sm_count / B)) : 1;
-    int tr = L.timer_begin(T_RERANK);
-    if (slices > 1) {
-        // Small batch: one CTA per query would leave most SMs idle (batch-1 latency).  Same two kernels as the
-        // host-driven multi-GPU path: cosines by `slices` CTAs per query, then the pool-wide fusion from the gathered cosines.
-        const size_t slots = size_t(B) * kRerankMaxCand;
+    const bool split = slices == 1 && ix->opt_rerank_mode != 0;
+    const size_t slots = size_t(B) * kRerankMaxCand;
+    if (slices > 1 || split) {                             // exchange arrays of the cosine and fuse kernels
         if ((rc = ws->r_split[0].ensure(sizeof(float) * slots * kRerankMaxChunks))) return rc;
         if ((rc = ws->r_split[1].ensure(sizeof(int32_t) * slots))) return rc;
         if ((rc = ws->r_split[2].ensure(sizeof(int64_t) * slots))) return rc;
         if ((rc = ws->r_split[3].ensure(sizeof(int32_t) * slots))) return rc;
         if ((rc = ws->r_split[4].ensure(sizeof(float) * slots))) return rc;
         if ((rc = ws->r_split[5].ensure(sizeof(int32_t) * size_t(B)))) return rc;
+    }
+    if (split && (rc = ws->r_units.ensure(sizeof(int32_t) * (size_t(B) + 2)))) return rc;
+    int tr = L.timer_begin(T_RERANK);
+    if (slices > 1) {
+        // Small batch: one CTA per query would leave most SMs idle (batch-1 latency).  Same two kernels as the
+        // host-driven multi-GPU path: cosines by `slices` CTAs per query, then the pool-wide fusion from the gathered cosines.
         MSE_CUDA_TRY(cudaMemsetAsync(ws->r_split[1].p, 0, sizeof(int32_t) * slots, st));      // rows: 0 = not fetched
         RerankShardArgs sa{a.cand_off, a.cand_count, a.cand_stride, a.cand_doc, a.cand_bm25, a.url_group, a.q, a.max_chunks,
                            int64_t(ix->dn.doc_base) + ix->dn.n_docs,
@@ -435,6 +442,24 @@ int rerank_enqueue(mse_index* ix, Lease& L, int32_t B, RerankArgs a) {
         rerank_shard_cos_kernel<<<dim3(unsigned(B), unsigned(slices)), kRerankThreads, 0, st>>>(ix->dn, sa);
         MSE_CUDA_TRY(cudaGetLastError());
         RerankFuseArgs fa{sa.cos, sa.rows, sa.chunk0, sa.surv_doc, sa.surv_bm25, sa.surv_count, a.smoothing, a.max_out,
+                          a.out_doc, a.out_score, a.out_orig, a.out_chunk, a.out_count, a.out_rows};
+        rerank_shard_fuse_kernel<<<B, kRerankThreads, 0, st>>>(fa);
+        MSE_CUDA_TRY(cudaGetLastError());
+    } else if (split) {
+        // Large batch (rerank_split.cuh): survivors per query, then one persistent grid streams the rows of all queries
+        // at the HBM roofline, then the fusion of rerank_shard_fuse_kernel.  Every array a kernel reads is written in full
+        // by the kernel before it: no memset.
+        RerankSplitBufs w{ws->r_split[0].as<float>(), ws->r_split[1].as<int32_t>(), ws->r_split[2].as<int64_t>(),
+                          ws->r_split[3].as<int32_t>(), ws->r_split[4].as<float>(), ws->r_split[5].as<int32_t>(),
+                          ws->r_units.as<int32_t>(), ws->r_units.as<int32_t>() + B + 1};
+        rerank_prep_kernel<<<B, kRerankThreads, 0, st>>>(ix->dn, a, w);
+        MSE_CUDA_TRY(cudaGetLastError());
+        rerank_units_scan_kernel<<<1, 1024, 0, st>>>(w.unit_off, B, w.next_unit);
+        MSE_CUDA_TRY(cudaGetLastError());
+        RerankGatherArgs ga{a.q, w.unit_off, w.next_unit, w.surv_count, w.rows, w.chunk0, w.cos, B};
+        rerank_gather_kernel<<<unsigned(ix->gather_ctas_per_sm * ix->sm_count), kRerankGatherThreads, 0, st>>>(ix->dn, ga);
+        MSE_CUDA_TRY(cudaGetLastError());
+        RerankFuseArgs fa{w.cos, w.rows, w.chunk0, w.surv_doc, w.surv_bm25, w.surv_count, a.smoothing, a.max_out,
                           a.out_doc, a.out_score, a.out_orig, a.out_chunk, a.out_count, a.out_rows};
         rerank_shard_fuse_kernel<<<B, kRerankThreads, 0, st>>>(fa);
         MSE_CUDA_TRY(cudaGetLastError());
@@ -523,6 +548,8 @@ int mse_index_create(int device, mse_index** out) {
         e = cudaFuncSetAttribute(bm25_score16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
         if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ix->score_ctas_per_sm[2], bm25_score16_kernel, kBm25Threads, smem);
     }
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ix->gather_ctas_per_sm, rerank_gather_kernel, kRerankGatherThreads, 0);
+    if (e == cudaSuccess && ix->gather_ctas_per_sm < 1) e = cudaErrorInvalidConfiguration;
     if (e != cudaSuccess) {
         set_error("kernel attribute setup failed: %s", cudaGetErrorString(e));
         (void)cudaGetLastError();
@@ -597,6 +624,7 @@ int mse_index_set_option(mse_index* ix, const char* name, int64_t value) {
     else if (!strcmp(name, "bm25_cand_cap")) ix->opt_cand_cap = value;
     else if (!strcmp(name, "bm25_use_tau")) ix->opt_use_tau = value;
     else if (!strcmp(name, "dense_scan_ctas_per_sm")) ix->opt_scan_ctas = value;
+    else if (!strcmp(name, "rerank_mode")) ix->opt_rerank_mode = value;                 // 1 (default): rerank_split.cuh kernels for batches past the small-batch split, 0: rerank_kernel
     else if (!strcmp(name, "dense_gemm_min_batch")) ix->opt_gemm_min_batch = value;
     else if (!strcmp(name, "dense_gemm_debug")) ix->opt_gemm_debug = value;
     else if (!strcmp(name, "dense_gemm_pair_mode")) ix->opt_gemm_pair_mode = value;     // 1 (default): multicast pair (cta_group::1), 2: cta_group::2 pair (measured slower: 4.7 vs 3.9 ms at C3 B=256)

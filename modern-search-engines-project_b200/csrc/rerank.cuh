@@ -48,7 +48,7 @@ __device__ __forceinline__ void block_bitonic_desc(uint64_t* buf, int P) {
     for (int k = 2; k <= P; k <<= 1) {
         for (int j = k >> 1; j > 0; j >>= 1) {
             for (int t = threadIdx.x; t < (P >> 1); t += NT) {
-                int i = ((t / j) * 2 * j) + (t % j);
+                const int i = ((t & ~(j - 1)) << 1) | (t & (j - 1));     // (t / j) * 2j + t % j: j is a power of two
                 int p = i + j;
                 uint64_t a = buf[i], b = buf[p];
                 bool up = ((i & k) == 0);
@@ -127,23 +127,31 @@ __device__ __forceinline__ int rerank_sort_dedupe(const int32_t* __restrict__ ca
         }
         __syncthreads();
     }
-    if (tid < 32) {                                        // stable compaction of the survivors (one warp)
-        int carry = 0;
-        for (int b0 = 0; b0 < P; b0 += 32) {
-            const int i = b0 + tid;
-            const uint64_t k = i < P ? s_key[i] : 0ull;
-            const int keep = ((k >> 63) && !s_dup[i]) ? 1 : 0;
-            const int incl = warp_incl_scan(keep);
-            __syncwarp();
-            if (keep) {
-                const int o = carry + incl - 1;
-                s_doc[o] = int32_t(0x7fffffffu - uint32_t((k >> 10) & 0x7fffffffu));
-                s_bm[o] = cand_bm25[0x3ff - int(k & 0x3ffull)];
-            }
-            carry += __shfl_sync(0xffffffffu, incl, 31);
+    // stable compaction of the survivors: warp w takes the slice [w * per, (w + 1) * per) and starts writing after the
+    // survivors of the slices before it
+    __shared__ int s_wcount[NT / 32];
+    const int per = (((P + NT / 32 - 1) / (NT / 32)) + 31) & ~31;
+    const int lo = warp_id() * per, hi = min(P, lo + per);
+    int cnt = 0;
+    for (int i = lo + lane_id(); i < hi; i += 32) cnt += ((s_key[i] >> 63) && !s_dup[i]) ? 1 : 0;
+    cnt = __reduce_add_sync(0xffffffffu, cnt);
+    if (lane_id() == 0) s_wcount[warp_id()] = cnt;
+    __syncthreads();
+    int carry = 0;
+    for (int w = 0; w < warp_id(); ++w) carry += s_wcount[w];
+    for (int b0 = lo; b0 < hi; b0 += 32) {
+        const int i = b0 + lane_id();
+        const uint64_t k = i < hi ? s_key[i] : 0ull;
+        const int keep = ((k >> 63) && !s_dup[i]) ? 1 : 0;
+        const int incl = warp_incl_scan(keep);
+        if (keep) {
+            const int o = carry + incl - 1;
+            s_doc[o] = int32_t(0x7fffffffu - uint32_t((k >> 10) & 0x7fffffffu));
+            s_bm[o] = cand_bm25[0x3ff - int(k & 0x3ffull)];
         }
-        if (tid == 0) *s_ns = carry;
+        carry += __shfl_sync(0xffffffffu, incl, 31);
     }
+    if (tid == NT - 1) *s_ns = carry;                      // the last warp ends where all survivors end
     __syncthreads();
     return *s_ns;
 }

@@ -123,7 +123,8 @@ struct RerankFuseArgs {
     int32_t* out_rows;
 };
 
-__global__ void __launch_bounds__(kRerankThreads)
+// 6 CTAs per SM (40 registers, a few spills to L1): 0.32 instead of 0.34 ms at 4 CTAs per SM for the large-batch rerank at C5
+__global__ void __launch_bounds__(kRerankThreads, 6)
 rerank_shard_fuse_kernel(RerankFuseArgs a) {
     constexpr int NT = kRerankThreads;
     __shared__ uint64_t s_key[kRerankMaxCand];
@@ -142,10 +143,12 @@ rerank_shard_fuse_kernel(RerankFuseArgs a) {
             T += n;
             const float bm = a.surv_bm25[base + i];
             bmin = fminf(bmin, bm); bmax = fmaxf(bmax, bm);
-            for (int j = 0; j < n; ++j) {
-                const float c = a.cos[(base + i) * kRerankMaxChunks + j];
-                cmin = fminf(cmin, c); cmax = fmaxf(cmax, c);
-            }
+#pragma unroll
+            for (int j = 0; j < kRerankMaxChunks; ++j)             // (unrolled: the row loads of a survivor are in flight together)
+                if (j < n) {
+                    const float c = a.cos[(base + i) * kRerankMaxChunks + j];
+                    cmin = fminf(cmin, c); cmax = fmaxf(cmax, c);
+                }
         }
     }
     cmin = block_reduce<NT>(cmin, s_tmp, 2);

@@ -69,7 +69,7 @@ struct Workspace {
     // dense scan
     DevBuf best, dq, overflow, qb16, log_key, log_q;
     // rerank
-    DevBuf r_in[4], r_out[6], r_split[6];
+    DevBuf r_in[4], r_out[6], r_split[6], r_units;
     // merge / shard exchange
     DevBuf m_in[3], x_recv, x_merge[4], x_surv, x_gath, x_cos, x_rows, x_own, x_mm, x_rtot, x_rec, x_rrecv;
 
