@@ -120,8 +120,6 @@ int mse_index_destroy(mse_index* idx);
  *   "dense_gemm_min_batch"   smallest batch routed to the tcgen05 GEMM kernel (default 8; faster from 3 on, but queries are rounded to bf16 there)
  *   "dense_gemm_pair_mode"   batches of 129..256 queries run as clusters of two CTAs: 1 (default) = every E tile TMA-multicast into
  *                            both CTAs, cta_group::1 MMAs; 2 = cta_group::2 MMAs issued by the leader CTA, E stages split
- *   "rerank_mode"            rerank of batches the small-batch split does not take: 1 (default) = prep, unit scan, persistent
- *                            gather and fuse kernels; 0 = one CTA per query (rerank_kernel).  Identical results
  *   "timers"                 1 (default) = bracket the kernels with CUDA events (mse_kernel_time), 0 = off
  *   "reset_timers"           any value: zero the accumulated kernel timers
  * Environment: MSE_DEBUG_SYNC=1 synchronises after every BM25 kernel so that a device fault names its kernel. */
@@ -219,7 +217,7 @@ int mse_dense_scan_batch_async(mse_index* idx, int32_t n_queries, const float* q
  *   cand_off[n_queries+1], cand_doc[], cand_bm25[]   candidates per query in BM25 order (GLOBAL dense index)
  *   url_group[n_docs] or NULL   id of the url-up-to-'?' group of each local doc (:44-47); among
  *       candidates of one group only the lowest doc survives; NULL = the groups stored by mse_dense_set_url_groups, if any
- *   q            float32 [n_queries*768], NOT normalised (:355)
+ *   q            float32 [n_queries*768], NOT normalised (:355); a device pointer must be 16-byte aligned
  *   out_*        [n_queries*max_out]: docs sorted by fused score descending; out_orig = min-max'd BM25
  *                score, out_chunk = global row (== chunk id) of the representative chunk,
  *                out_rows[n_queries] = fetched chunk rows (`total_documents` of the reference response).
@@ -232,7 +230,8 @@ int mse_rerank_batch(mse_index* idx, int32_t n_queries, const int32_t* cand_off,
 
 /* One hybrid query batch: BM25 top_k candidates (:252 `bm_25.search(query, top_k=1000)`) handed on the device to the
  * rerank stage (:259-274) -> max_out results per query.  Inputs as mse_bm25_search_batch_async (q_off / q_term / q_tf,
- * n_slots) plus q_vec float32 [n_queries*768]; outputs as mse_rerank_batch.  top_k <= MSE_MAX_RERANK_CAND.
+ * n_slots) plus q_vec float32 [n_queries*768] (16-byte aligned on the device); outputs as mse_rerank_batch.
+ * top_k <= MSE_MAX_RERANK_CAND.
  * `where` = MSE_HOST (exact, complete on return), MSE_DEVICE or MSE_HOST_ASYNC (enqueue-only, see `status`). */
 int mse_hybrid_search_batch(mse_index* idx, int32_t n_queries, int32_t n_slots, const int32_t* q_off,
                             const int32_t* q_term, const int32_t* q_tf, const float* q_vec,
@@ -241,7 +240,7 @@ int mse_hybrid_search_batch(mse_index* idx, int32_t n_queries, int32_t n_slots, 
                             int32_t* out_count, int32_t* out_rows, int32_t* status, int where, void* stream);
 
 /* Sharded form of mse_rerank_batch, host-driven variant (chunk table sharded by doc range over several GPUs);
- * device buffers only.  Step 1, every rank: same replicated candidates; dedupes, then fills the cosines of the
+ * device buffers only (q 16-byte aligned).  Step 1, every rank: same replicated candidates; dedupes, then fills the cosines of the
  * candidates whose documents THIS shard owns into cos[B][1024][10] / rows[B][1024] / chunk0[B][1024] (zeroed here
  * first) and the replicated survivor description surv_*.  url_group is indexed by the GLOBAL dense doc index.
  * The caller then sums cos / rows / chunk0 over the ranks and calls step 2 on any rank.  (mse_hybrid_search_sharded
@@ -295,7 +294,7 @@ int mse_bm25_search_sharded(mse_index* idx, int32_t n_queries, int32_t n_slots, 
  *   4. all-reduce(min, max) of 4 floats per query: the pool-wide normalisation bounds of :289-296
  *   5. every rank: fusion + positional weighting + per-doc max of ITS documents (:299-372), local top max_out
  *   6. the local lists travel to the query owner, which merges them: scores are formed exactly as on one GPU.
- * q_vec float32 [n_queries*768].  Outputs as mse_rerank_batch for the queries_per_rank owned queries. */
+ * q_vec float32 [n_queries*768], 16-byte aligned.  Outputs as mse_rerank_batch for the queries_per_rank owned queries. */
 int mse_hybrid_search_sharded(mse_index* idx, int32_t n_queries, int32_t n_slots, const int32_t* q_off,
                               const int32_t* q_term, const int32_t* q_tf, const float* q_vec,
                               int32_t top_k, float min_score, int32_t shard_list_len,

@@ -70,7 +70,6 @@ struct mse_index {
     int64_t stats[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     std::atomic<int> u16_backoff{0};              // calls the fp32 score kernel still serves after a hostile batch (bm25_enqueue)
     int score_ctas_per_sm[3] = {0, 0, 0};         // occupancy of the score kernel (fp32 scan / fp32 hit read-out / two-phase) at its default range
-    int64_t opt_rerank_mode = 1;                  // batches past the small-batch split: 0 = rerank_kernel, 1 = prep / gather / fuse kernels
     int gather_ctas_per_sm = 0;                   // occupancy of rerank_gather_kernel (its persistent grid)
 };
 
@@ -98,6 +97,8 @@ int copy_out(void* dst, const void* src, size_t bytes, cudaStream_t s) {
     return MSE_OK;
 }
 bool is_host(int where) { return where == MSE_HOST || where == MSE_HOST_ASYNC; }
+// the rerank kernels read query vectors as float4 (rerank_query_frag)
+bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 int round_up(int64_t v, int64_t m) { return int(((v + m - 1) / m) * m); }
 
@@ -419,17 +420,15 @@ int rerank_enqueue(mse_index* ix, Lease& L, int32_t B, RerankArgs a) {
     int rc;
     if (!a.url_group && ix->n_url_groups >= ix->dn.n_docs && ix->dn.doc_base == 0 && ix->n_url_groups > 0) a.url_group = ix->url_group.as<int32_t>();
     const int slices = (B * 4 <= ix->sm_count && ix->dn.doc_base == 0) ? std::min(32, std::max(1, ix->sm_count / B)) : 1;
-    const bool split = slices == 1 && ix->opt_rerank_mode != 0;
     const size_t slots = size_t(B) * kRerankMaxCand;
-    if (slices > 1 || split) {                             // exchange arrays of the cosine and fuse kernels
-        if ((rc = ws->r_split[0].ensure(sizeof(float) * slots * kRerankMaxChunks))) return rc;
-        if ((rc = ws->r_split[1].ensure(sizeof(int32_t) * slots))) return rc;
-        if ((rc = ws->r_split[2].ensure(sizeof(int64_t) * slots))) return rc;
-        if ((rc = ws->r_split[3].ensure(sizeof(int32_t) * slots))) return rc;
-        if ((rc = ws->r_split[4].ensure(sizeof(float) * slots))) return rc;
-        if ((rc = ws->r_split[5].ensure(sizeof(int32_t) * size_t(B)))) return rc;
-    }
-    if (split && (rc = ws->r_units.ensure(sizeof(int32_t) * (size_t(B) + 2)))) return rc;
+    // exchange arrays between the cosine (or prep and gather) kernels and the fuse kernel
+    if ((rc = ws->r_split[0].ensure(sizeof(float) * slots * kRerankMaxChunks))) return rc;
+    if ((rc = ws->r_split[1].ensure(sizeof(int32_t) * slots))) return rc;
+    if ((rc = ws->r_split[2].ensure(sizeof(int64_t) * slots))) return rc;
+    if ((rc = ws->r_split[3].ensure(sizeof(int32_t) * slots))) return rc;
+    if ((rc = ws->r_split[4].ensure(sizeof(float) * slots))) return rc;
+    if ((rc = ws->r_split[5].ensure(sizeof(int32_t) * size_t(B)))) return rc;
+    if (slices == 1 && (rc = ws->r_units.ensure(sizeof(int32_t) * (size_t(B) + 2)))) return rc;
     int tr = L.timer_begin(T_RERANK);
     if (slices > 1) {
         // Small batch: one CTA per query would leave most SMs idle (batch-1 latency).  Same two kernels as the
@@ -445,7 +444,7 @@ int rerank_enqueue(mse_index* ix, Lease& L, int32_t B, RerankArgs a) {
                           a.out_doc, a.out_score, a.out_orig, a.out_chunk, a.out_count, a.out_rows};
         rerank_shard_fuse_kernel<<<B, kRerankThreads, 0, st>>>(fa);
         MSE_CUDA_TRY(cudaGetLastError());
-    } else if (split) {
+    } else {
         // Large batch (rerank_split.cuh): survivors per query, then one persistent grid streams the rows of all queries
         // at the HBM roofline, then the fusion of rerank_shard_fuse_kernel.  Every array a kernel reads is written in full
         // by the kernel before it: no memset.
@@ -462,9 +461,6 @@ int rerank_enqueue(mse_index* ix, Lease& L, int32_t B, RerankArgs a) {
         RerankFuseArgs fa{w.cos, w.rows, w.chunk0, w.surv_doc, w.surv_bm25, w.surv_count, a.smoothing, a.max_out,
                           a.out_doc, a.out_score, a.out_orig, a.out_chunk, a.out_count, a.out_rows};
         rerank_shard_fuse_kernel<<<B, kRerankThreads, 0, st>>>(fa);
-        MSE_CUDA_TRY(cudaGetLastError());
-    } else {
-        rerank_kernel<<<B, kRerankThreads, kRerankSmemBytes, st>>>(ix->dn, a);
         MSE_CUDA_TRY(cudaGetLastError());
     }
     L.timer_end(tr);
@@ -533,8 +529,7 @@ int mse_index_create(int device, mse_index** out) {
     ix->device = device;
     ix->sm_count = prop.multiProcessorCount;
     // function attributes are set once here, so that no search call touches them (calls may run inside a stream capture)
-    cudaError_t e = cudaFuncSetAttribute(rerank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kRerankSmemBytes));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(dense_gemm_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kGemmSmemBytes));
+    cudaError_t e = cudaFuncSetAttribute(dense_gemm_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kGemmSmemBytes));
     if (e == cudaSuccess) e = cudaFuncSetAttribute(dense_gemm_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kGemmSmemBytes));
     if (e == cudaSuccess) e = cudaFuncSetAttribute(dense_gemm_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kGemmSmemBytes));
     for (int hits = 0; hits < 2 && e == cudaSuccess; ++hits) {
@@ -624,7 +619,6 @@ int mse_index_set_option(mse_index* ix, const char* name, int64_t value) {
     else if (!strcmp(name, "bm25_cand_cap")) ix->opt_cand_cap = value;
     else if (!strcmp(name, "bm25_use_tau")) ix->opt_use_tau = value;
     else if (!strcmp(name, "dense_scan_ctas_per_sm")) ix->opt_scan_ctas = value;
-    else if (!strcmp(name, "rerank_mode")) ix->opt_rerank_mode = value;                 // 1 (default): rerank_split.cuh kernels for batches past the small-batch split, 0: rerank_kernel
     else if (!strcmp(name, "dense_gemm_min_batch")) ix->opt_gemm_min_batch = value;
     else if (!strcmp(name, "dense_gemm_debug")) ix->opt_gemm_debug = value;
     else if (!strcmp(name, "dense_gemm_pair_mode")) ix->opt_gemm_pair_mode = value;     // 1 (default): multicast pair (cta_group::1), 2: cta_group::2 pair (measured slower: 4.7 vs 3.9 ms at C3 B=256)
@@ -1307,6 +1301,7 @@ int mse_rerank_batch(mse_index* ix, int32_t B, const int32_t* cand_off, const in
     MSE_REQUIRE(where == MSE_HOST || where == MSE_DEVICE || where == MSE_HOST_ASYNC, "bad `where`");
     MSE_REQUIRE(B >= 0 && cand_off && out_count && out_rows, "null/negative argument");
     MSE_REQUIRE(B == 0 || (q && out_doc && out_score && out_orig && out_chunk), "null argument");
+    MSE_REQUIRE(is_host(where) || aligned16(q), "device query vectors must be 16-byte aligned");
     if (max_chunks < 1 || max_chunks > kRerankMaxChunks) { set_error("max_chunks %d outside [1, %d]", max_chunks, kRerankMaxChunks); return MSE_ERR_UNSUPPORTED; }
     if (max_out < 1 || max_out > kRerankMaxCand) { set_error("max_out %d outside [1, %d]", max_out, kRerankMaxCand); return MSE_ERR_UNSUPPORTED; }
     MSE_REQUIRE(smoothing >= 0.f && smoothing <= 1.f, "smoothing outside [0,1]");
@@ -1365,6 +1360,7 @@ int mse_hybrid_search_batch(mse_index* ix, int32_t B, int32_t S, const int32_t* 
     MSE_REQUIRE(where == MSE_HOST || where == MSE_DEVICE || where == MSE_HOST_ASYNC, "bad `where`");
     MSE_REQUIRE(B >= 0 && S >= 0 && q_off && out_count && out_rows && (S == 0 || (q_term && q_tf)), "null/negative argument");
     MSE_REQUIRE(B == 0 || (q_vec && out_doc && out_score && out_orig && out_chunk), "null argument");
+    MSE_REQUIRE(is_host(where) || aligned16(q_vec), "device query vectors must be 16-byte aligned");
     if (top_k < 1 || top_k > kRerankMaxCand) { set_error("top_k %d outside [1, %d]", top_k, kRerankMaxCand); return MSE_ERR_UNSUPPORTED; }
     if (max_chunks < 1 || max_chunks > kRerankMaxChunks) { set_error("max_chunks %d outside [1, %d]", max_chunks, kRerankMaxChunks); return MSE_ERR_UNSUPPORTED; }
     if (max_out < 1 || max_out > kRerankMaxCand) { set_error("max_out %d outside [1, %d]", max_out, kRerankMaxCand); return MSE_ERR_UNSUPPORTED; }
@@ -1442,6 +1438,7 @@ int mse_rerank_shard_cos(mse_index* ix, int32_t B, const int32_t* cand_off, cons
     if (!ix) { set_error("null index"); return MSE_ERR_INVALID; }
     MSE_REQUIRE(B >= 0 && cand_off && cos && rows && chunk0 && surv_doc && surv_bm25 && surv_count, "null/negative argument");
     MSE_REQUIRE(B == 0 || (q && cand_doc && cand_bm25), "null argument");
+    MSE_REQUIRE(aligned16(q), "device query vectors must be 16-byte aligned");
     if (max_chunks < 1 || max_chunks > kRerankMaxChunks) { set_error("max_chunks %d outside [1, %d]", max_chunks, kRerankMaxChunks); return MSE_ERR_UNSUPPORTED; }
     if (!ix->has_dense) { set_error("mse_dense_load has not been called"); return MSE_ERR_STATE; }
     if (B == 0) return MSE_OK;
@@ -1661,6 +1658,7 @@ int mse_hybrid_search_sharded(mse_index* ix, int32_t GB, int32_t S, const int32_
     if (!ix) { set_error("null index"); return MSE_ERR_INVALID; }
     MSE_REQUIRE(GB >= 0 && S >= 0 && q_off && out_count && out_rows && (S == 0 || (q_term && q_tf)), "null/negative argument");
     MSE_REQUIRE(GB == 0 || (q_vec && out_doc && out_score && out_orig && out_chunk), "null argument");
+    MSE_REQUIRE(aligned16(q_vec), "device query vectors must be 16-byte aligned");
     if (top_k < 1 || top_k > kRerankMaxCand) { set_error("top_k %d outside [1, %d]", top_k, kRerankMaxCand); return MSE_ERR_UNSUPPORTED; }
     if (max_chunks < 1 || max_chunks > kRerankMaxChunks) { set_error("max_chunks %d outside [1, %d]", max_chunks, kRerankMaxChunks); return MSE_ERR_UNSUPPORTED; }
     if (max_out < 1 || max_out > kRerankMaxCand) { set_error("max_out %d outside [1, %d]", max_out, kRerankMaxCand); return MSE_ERR_UNSUPPORTED; }

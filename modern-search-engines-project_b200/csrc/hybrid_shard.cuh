@@ -13,8 +13,9 @@
 //   hyb_fuse_kernel    every rank, every query: min-max, 0.85/0.15 fusion, positional weighting, per-doc max of ITS
 //                      documents, sort, local top max_out as records {key, chunk, orig}  --- records travel to the owner ---
 //   hyb_final_kernel   owner: merge of the W sorted record lists by rank counting (no sort), write-out.
-// A document's fused score is formed on exactly one rank from the global bounds with the same operations as
-// rerank_kernel, so the result equals the single-GPU result.
+// A document's cosines and fused score are formed on exactly one rank from the global bounds with the helpers of the
+// single-GPU kernels (rerank_query_frag, rerank_row_dot, rerank_cos, rerank_fuse_doc), so the result equals the single-GPU
+// result.
 #pragma once
 #include "common.cuh"
 #include "dense.cuh"
@@ -103,21 +104,11 @@ hyb_cos_kernel(DenseDev dx, HybCosArgs a) {
     if (blockIdx.y == 0 && threadIdx.x == 0) a.own[qi] = make_int2(lo, hi);
     if (lo >= hi) return;
     const int max_chunks = a.max_chunks < kRerankMaxChunks ? a.max_chunks : kRerankMaxChunks;
-    const float* qv = a.q + int64_t(qi) * kDim;
     float qf[24];
-    float qq = 0.f;
-#pragma unroll
-    for (int j = 0; j < 3; ++j)
-#pragma unroll
-        for (int e = 0; e < 8; ++e) {
-            qf[j * 8 + e] = qv[j * 256 + lane_id() * 8 + e];
-            qq = fmaf(qf[j * 8 + e], qf[j * 8 + e], qq);
-        }
-    qq = warp_sum(qq);
-    const float qn = sqrtf(qq);
+    const float qn = rerank_query_frag(a.q + int64_t(qi) * kDim, qf);
     float cmin = INFINITY, cmax = -INFINITY, bmin = INFINITY, bmax = -INFINITY;
     int rows_here = 0;
-    constexpr int RIF = 5;                                   // rows in flight per warp, as rerank_kernel
+    constexpr int RIF = 5;                                   // rows in flight per warp
     for (int i = lo + int(blockIdx.y) * (NT / 32) + warp_id(); i < hi; i += int(gridDim.y) * (NT / 32)) {
         const uint64_t sv = surv[i];
         const int64_t d = int64_t(sv >> 32) - int64_t(dx.doc_base);
@@ -151,20 +142,9 @@ hyb_cos_kernel(DenseDev dx, HybCosArgs a) {
 #pragma unroll
             for (int k = 0; k < RIF; ++k) {
                 if ((b + k) >= n) break;                   // uniform
-                float dot = 0.f;
-#pragma unroll
-                for (int j = 0; j < 3; ++j) {
-                    float f[8];
-                    bf16x8_to_float(v[k][j], f);
-#pragma unroll
-                    for (int e = 0; e < 8; ++e) dot = fmaf(f[e], qf[j * 8 + e], dot);
-                }
-                dot = warp_sum(dot);
-                if ((b + k) < n) {
-                    const float c = dot / (sqrtf(ee[k]) * qn);
-                    cmin = fminf(cmin, c); cmax = fmaxf(cmax, c);
-                    if (lane_id() == 0) a.cos[slot * kRerankMaxChunks + b + k] = c;
-                }
+                const float c = rerank_cos(rerank_row_dot(v[k], qf), ee[k], qn);
+                cmin = fminf(cmin, c); cmax = fmaxf(cmax, c);
+                if (lane_id() == 0) a.cos[slot * kRerankMaxChunks + b + k] = c;
             }
         }
     }
@@ -226,22 +206,8 @@ hyb_fuse_kernel(DenseDev dx, HybFuseArgs a) {
         if (n > 0) {
             const uint64_t sv = surv[own.x + i];
             const double oldn = brange == 0.0 ? 0.0 : (double(__uint_as_float(uint32_t(sv))) - double(bmin)) / brange;
-            double vals[kRerankMaxChunks];
-            double best = -1.0;
-            int bi = 0;
-            for (int j = 0; j < n; ++j) {
-                const double cn = crange == 0.0 ? 0.0 : (double(a.cos[slot * kRerankMaxChunks + j]) - double(cmin)) / crange;
-                vals[j] = cn * (1.0 - sm) + oldn * sm;
-                if (vals[j] > best) { best = vals[j]; bi = j; }
-            }
-            if (n > 1) {
-                const double adj = 0.1 - (0.1 + 0.05) * (double(bi) / double(n - 1));
-                double v = vals[bi] + adj;
-                vals[bi] = v < 0.0 ? 0.0 : (v > 1.0 ? 1.0 : v);
-                best = -1.0;
-                for (int j = 0; j < n; ++j) if (vals[j] > best) { best = vals[j]; bi = j; }
-            }
-            const float sc = float(best) + 0.0f;
+            int bi;
+            const float sc = rerank_fuse_doc(a.cos + slot * kRerankMaxChunks, n, oldn, double(cmin), crange, sm, &bi);
             key = make_key64(float_to_key(sc), uint32_t(sv >> 32));       // score desc, doc asc
             s_orig[i] = float(oldn); s_best[i] = uint8_t(bi);
         }

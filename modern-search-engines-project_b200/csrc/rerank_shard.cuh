@@ -11,7 +11,7 @@
 //   rerank_shard_fuse_kernel  pool-wide min-max, 0.85/0.15 fusion, positional weighting, per-doc max, sort
 //                             (:299-372) from the gathered cosines — no embedding access, same result on
 //                             every rank.
-// On one GPU the fused rerank_kernel (rerank.cuh) does all of this in one pass.
+// On one GPU, small batches run the same two kernels (rerank_enqueue in api.cu, with a 2-D cosine grid and no exchange).
 #pragma once
 #include "common.cuh"
 #include "dense.cuh"
@@ -50,11 +50,8 @@ rerank_shard_cos_kernel(DenseDev dx, RerankShardArgs a) {
     __shared__ int s_ns;
     const int qi = blockIdx.x;
     const int tid = threadIdx.x;
-    int c0, nc;
-    if (a.cand_off) { c0 = a.cand_off[qi]; nc = a.cand_off[qi + 1] - c0; }
-    else { c0 = qi * a.cand_stride; nc = a.cand_count[qi]; }
-    if (nc < 0) nc = 0;
-    if (nc > kRerankMaxCand) nc = kRerankMaxCand;
+    int c0;
+    const int nc = rerank_query_range(a.cand_off, a.cand_count, a.cand_stride, qi, &c0);
     // ascending (doc, input slot), URL-group dedupe; docs outside [0, n_docs_global) are dropped (-1 padding of BM25 results)
     rerank_sort_dedupe<NT>(a.cand_doc + c0, a.cand_bm25 + c0, nc, 0, a.n_docs_global, a.url_group,
                            s_key, s_key2, s_dup, s_doc, s_bm, &s_ns);
@@ -69,18 +66,8 @@ rerank_shard_cos_kernel(DenseDev dx, RerankShardArgs a) {
     const int max_chunks = a.max_chunks < kRerankMaxChunks ? a.max_chunks : kRerankMaxChunks;
 
     // cosines of the rows this rank owns: one warp per (survivor, chunk) row
-    const float* qv = a.q + int64_t(qi) * kDim;
     float qf[24];
-    float qq = 0.f;
-#pragma unroll
-    for (int j = 0; j < 3; ++j)
-#pragma unroll
-        for (int e = 0; e < 8; ++e) {
-            qf[j * 8 + e] = qv[j * 256 + lane_id() * 8 + e];
-            qq = fmaf(qf[j * 8 + e], qf[j * 8 + e], qq);
-        }
-    qq = warp_sum(qq);
-    const float qn = sqrtf(qq);
+    const float qn = rerank_query_frag(a.q + int64_t(qi) * kDim, qf);
     // gridDim.y > 1 (small batches on one GPU): the survivors of a query are dealt out to gridDim.y CTAs
     for (int i = int(blockIdx.y) * (NT / 32) + warp_id(); i < ns; i += int(gridDim.y) * (NT / 32)) {
         const int64_t d = int64_t(s_doc[i]) - int64_t(dx.doc_base);
@@ -91,17 +78,11 @@ rerank_shard_cos_kernel(DenseDev dx, RerankShardArgs a) {
         if (lane_id() == 0) { a.rows[slot] = n; a.chunk0[slot] = dx.chunk_base + ra; }
         for (int j = 0; j < n; ++j) {
             const uint4* p = reinterpret_cast<const uint4*>(dx.emb + (ra + j) * kDim) + lane_id();
-            float dot = 0.f;
-            const float ee = __ldg(dx.row_sq + ra + j);    // squared norm of the row, formed at load
+            uint4 v[3];
 #pragma unroll
-            for (int t = 0; t < 3; ++t) {
-                float f[8];
-                bf16x8_to_float(ldg_stream(p + t * 32), f);
-#pragma unroll
-                for (int e = 0; e < 8; ++e) dot = fmaf(f[e], qf[t * 8 + e], dot);
-            }
-            dot = warp_sum(dot);
-            if (lane_id() == 0) a.cos[slot * kRerankMaxChunks + j] = dot / (sqrtf(ee) * qn);
+            for (int t = 0; t < 3; ++t) v[t] = ldg_stream(p + t * 32);
+            const float c = rerank_cos(rerank_row_dot(v, qf), __ldg(dx.row_sq + ra + j), qn);
+            if (lane_id() == 0) a.cos[slot * kRerankMaxChunks + j] = c;
         }
     }
 }
@@ -173,22 +154,8 @@ rerank_shard_fuse_kernel(RerankFuseArgs a) {
         const int n = i < ns ? a.rows[base + i] : 0;
         if (n > 0) {
             const double oldn = brange == 0.0 ? 0.0 : (double(a.surv_bm25[base + i]) - double(bmin)) / brange;
-            double vals[kRerankMaxChunks];
-            double best = -1.0;
-            int bi = 0;
-            for (int j = 0; j < n; ++j) {
-                const double cn = crange == 0.0 ? 0.0 : (double(a.cos[(base + i) * kRerankMaxChunks + j]) - double(cmin)) / crange;
-                vals[j] = cn * (1.0 - sm) + oldn * sm;
-                if (vals[j] > best) { best = vals[j]; bi = j; }
-            }
-            if (n > 1) {
-                const double adj = 0.1 - (0.1 + 0.05) * (double(bi) / double(n - 1));
-                double v = vals[bi] + adj;
-                vals[bi] = v < 0.0 ? 0.0 : (v > 1.0 ? 1.0 : v);
-                best = -1.0;
-                for (int j = 0; j < n; ++j) if (vals[j] > best) { best = vals[j]; bi = j; }
-            }
-            const float sc = float(best) + 0.0f;
+            int bi;
+            const float sc = rerank_fuse_doc(a.cos + (base + i) * kRerankMaxChunks, n, oldn, double(cmin), crange, sm, &bi);
             key = (uint64_t(float_to_key(sc)) << 32) | (uint64_t(0x3fffffu - uint32_t(i)) << 10) | uint64_t(i);
             s_score[i] = sc; s_orig[i] = float(oldn); s_best[i] = uint8_t(bi);
         }

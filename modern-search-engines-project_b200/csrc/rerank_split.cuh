@@ -1,6 +1,6 @@
-// K5, large batches on one GPU: the rerank of rerank_kernel (rerank.cuh) split so that the row gather streams at the
-// HBM roofline.  rerank_kernel runs one CTA per query, and its sort / dedupe, row prefix, reductions, fusion and final
-// sort are phases with no bytes in flight; at 3 CTAs per SM those phases line up and leave HBM idle.  Here:
+// K5, large batches on one GPU, split so that the row gather streams at the HBM roofline.  With one CTA per query, the
+// sort / dedupe, row prefix, reductions, fusion and final sort are phases with no bytes in flight; at 3 CTAs per SM those
+// phases line up and leave HBM idle.  Here:
 //   rerank_prep_kernel        one CTA per query: sort + URL-group dedupe (rerank_sort_dedupe, unchanged), rows per
 //                             survivor, the survivor arrays rerank_shard_fuse_kernel reads, and the query's number of
 //                             work units (kRerankUnit consecutive survivors each)
@@ -8,8 +8,8 @@
 //   rerank_gather_kernel      persistent warps, no shared memory: a warp takes units from an atomic counter and streams
 //                             their rows with the next rows always in flight; cosines to cos[query][survivor][chunk]
 //   rerank_shard_fuse_kernel  pool-wide min-max, fusion, positional weighting, per-doc max, sort (rerank_shard.cuh)
-// Every cosine is formed with the arithmetic of rerank_kernel (same per-lane 3 x 8 striding, fmaf order, warp_sum, row
-// norm from DenseDev::row_sq, qn), and the fuse kernel repeats its fusion, so the outputs are bit-identical.
+// The cosines come from rerank_query_frag, rerank_row_dot and rerank_cos, the fusion from rerank_fuse_doc (rerank.cuh):
+// the outputs are bit-identical to those of the small-batch path.
 #pragma once
 #include "common.cuh"
 #include "dense.cuh"
@@ -44,11 +44,8 @@ rerank_prep_kernel(DenseDev dx, RerankArgs a, RerankSplitBufs w) {
     __shared__ int s_ns;
     const int qi = blockIdx.x;
     const int tid = threadIdx.x;
-    int c0, nc;
-    if (a.cand_off) { c0 = a.cand_off[qi]; nc = a.cand_off[qi + 1] - c0; }
-    else { c0 = qi * a.cand_stride; nc = a.cand_count[qi]; }
-    if (nc < 0) nc = 0;
-    if (nc > kRerankMaxCand) nc = kRerankMaxCand;
+    int c0;
+    const int nc = rerank_query_range(a.cand_off, a.cand_count, a.cand_stride, qi, &c0);
     const int ns = rerank_sort_dedupe<NT>(a.cand_doc + c0, a.cand_bm25 + c0, nc, int64_t(dx.doc_base), dx.n_docs, a.url_group,
                                           s_key, s_key2, s_dup, s_doc, s_bm, &s_ns);
     const int max_chunks = a.max_chunks < kRerankMaxChunks ? a.max_chunks : kRerankMaxChunks;
@@ -163,39 +160,18 @@ rerank_gather_kernel(DenseDev dx, RerankGatherArgs a) {
 #pragma unroll
         for (int s = 0; s < D; ++s)
             if (s < R) issue(s, s);
-        // query fragment and norm, exactly as rerank_kernel forms them
-        const float* qv = a.q + int64_t(qi) * kDim;
         float qf[24];
-        float qq = 0.f;
-#pragma unroll
-        for (int j = 0; j < 3; ++j) {
-            const float4 x = *reinterpret_cast<const float4*>(qv + j * 256 + lane * 8);
-            const float4 y = *reinterpret_cast<const float4*>(qv + j * 256 + lane * 8 + 4);
-            qf[j * 8 + 0] = x.x; qf[j * 8 + 1] = x.y; qf[j * 8 + 2] = x.z; qf[j * 8 + 3] = x.w;
-            qf[j * 8 + 4] = y.x; qf[j * 8 + 5] = y.y; qf[j * 8 + 6] = y.z; qf[j * 8 + 7] = y.w;
-        }
-#pragma unroll
-        for (int e = 0; e < 24; ++e) qq = fmaf(qf[e], qf[e], qq);
-        qq = warp_sum(qq);
-        const float qn = sqrtf(qq);
+        const float qn = rerank_query_frag(a.q + int64_t(qi) * kDim, qf);
 
         float* out = a.cos + slot0 * kRerankMaxChunks;
         for (int t0 = 0; t0 < R; t0 += D) {
 #pragma unroll
             for (int s = 0; s < D; ++s) {
                 if (t0 + s >= R) break;                    // uniform
-                float dot = 0.f;
-#pragma unroll
-                for (int j = 0; j < 3; ++j) {
-                    float f[8];
-                    bf16x8_to_float(v[s][j], f);
-#pragma unroll
-                    for (int e = 0; e < 8; ++e) dot = fmaf(f[e], qf[j * 8 + e], dot);
-                }
-                dot = warp_sum(dot);
+                const float dot = rerank_row_dot(v[s], qf);
                 int k, j;
                 locate(t0 + s, k, j);
-                if (lane == 0) out[k * kRerankMaxChunks + j] = dot / (sqrtf(ee[s]) * qn);
+                if (lane == 0) out[k * kRerankMaxChunks + j] = rerank_cos(dot, ee[s], qn);
                 if (t0 + s + D < R) issue(s, t0 + s + D);
             }
         }

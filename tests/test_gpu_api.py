@@ -148,7 +148,7 @@ def _stagewise(nat, q_off, q_term, q_tf, qv, top_k, max_out):
     return nat.rerank(cand_off, cd, cs, qv, None, 0.15, 10, max_out), (doc, score, count)
 
 
-@pytest.mark.parametrize("B", [3, 200])      # small batch: split rerank path; large: one CTA per query
+@pytest.mark.parametrize("B", [3, 200])      # small batch: 2-D cosine grid + fuse kernel; large: prep / gather / fuse kernels
 def test_hybrid_call_equals_the_two_stages_and_the_oracle(hybrid_index, B):
     h = hybrid_index
     nat, c, ix = h["nat"], h["c"], h["ix"]

@@ -1,6 +1,8 @@
 """GPU tests of the large-batch rerank (csrc/rerank_split.cuh: prep, unit scan, persistent gather, fuse kernels) against
-the fused one-CTA-per-query rerank_kernel, which `rerank_mode = 0` selects: all six outputs (doc, score, orig, chunk,
-count, rows) must be identical bit for bit, through every call form."""
+the small-batch path (rerank_shard_cos_kernel on a 2-D grid, then rerank_shard_fuse_kernel), which a batch of at most
+multi_processor_count // 4 queries takes on an index with doc_base 0.  The reference is the same call in such
+sub-batches; all six outputs (doc, score, orig, chunk, count, rows) must be identical bit for bit, through every call
+form."""
 import numpy as np
 import pytest
 import torch
@@ -64,13 +66,21 @@ def _sizes(B, seed):
     return s
 
 
-def _both(nat, *args, **kw):
-    nat.set_option("rerank_mode", 0)
-    try:
-        ref = nat.rerank(*args, **kw)
-    finally:
-        nat.set_option("rerank_mode", 1)
-    return ref, nat.rerank(*args, **kw)
+def _small_batch():
+    return torch.cuda.get_device_properties(0).multi_processor_count // 4
+
+
+def _small_batch_rerank(nat, off, cd, cs, q, *args):
+    """nat.rerank on consecutive sub-batches that each take the small-batch path, outputs concatenated."""
+    parts = []
+    for b0 in range(0, len(off) - 1, _small_batch()):
+        b1 = min(b0 + _small_batch(), len(off) - 1)
+        parts.append(nat.rerank(off[b0:b1 + 1] - off[b0], cd[off[b0]:off[b1]], cs[off[b0]:off[b1]], q[b0:b1], *args))
+    return tuple(np.concatenate(p) for p in zip(*parts))
+
+
+def _both(nat, *args):
+    return _small_batch_rerank(nat, *args), nat.rerank(*args)
 
 
 def _assert_same(got, ref):
@@ -82,7 +92,7 @@ def _assert_same(got, ref):
 
 @pytest.mark.parametrize("groups", [False, True])
 @pytest.mark.parametrize("max_chunks,max_out", [(10, 100), (10, 1), (3, 1024), (7, 100)])
-def test_split_equals_fused_kernel(corpus, groups, max_chunks, max_out):
+def test_split_equals_small_batch_path(corpus, groups, max_chunks, max_out):
     """1100 queries: the large-batch path.  max_out 1024 is more than any query's survivors."""
     c = corpus
     nat = c["nat"]
@@ -119,7 +129,9 @@ def test_split_queries_without_rows_and_duplicate_only_lists(corpus):
 
 def test_split_doc_base_shard(corpus):
     """A shard that starts at doc 3000 / chunk row off[3000]: global candidate ids, ids of other shards dropped; the
-    split path also takes small batches here (the small-batch split needs doc_base 0)."""
+    split path also takes small batches here (the small-batch split needs doc_base 0).  Reference: the corpus-wide index
+    in small batches, on the same lists with every id outside the shard replaced by -1 (which keeps each candidate's
+    input slot, the tie-break of the dedupe)."""
     c = corpus
     lo, hi = 3000, 9000
     off = c["off"]
@@ -131,8 +143,10 @@ def test_split_doc_base_shard(corpus):
         for B in (3, 600):
             co, cd, cs = _candidates(c["n_docs"], _sizes(B, 11 + B), 12 + B)    # most ids fall outside the shard
             q = synthetic.make_query_vectors(B, seed=13 + B)
+            cd_in = np.where((cd >= lo) & (cd < hi), cd, -1).astype(np.int32)
             for g in (None, grp):
-                ref, got = _both(sh, co, cd, cs, q, g, 0.15, 10, 100)
+                ref = _small_batch_rerank(c["nat"], co, cd_in, cs, q, None if g is None else c["grp"], 0.15, 10, 100)
+                got = sh.rerank(co, cd, cs, q, g, 0.15, 10, 100)
                 _assert_same(got, ref)
                 n = ref[4]
                 assert n.max() > 0
@@ -149,9 +163,7 @@ def test_split_device_calls_and_graph_capture(corpus):
     B = 1024
     off, cd, cs = _candidates(c["n_docs"], _sizes(B, 21), 22)
     q = synthetic.make_query_vectors(B, seed=23)
-    nat.set_option("rerank_mode", 0)
-    ref = nat.rerank(off, cd, cs, q, c["grp"], 0.15, 10, 100)
-    nat.set_option("rerank_mode", 1)
+    ref = _small_batch_rerank(nat, off, cd, cs, q, c["grp"], 0.15, 10, 100)
     t = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(DEV)
     d = (t(off), t(cd), t(cs), t(q), t(c["grp"]))
     got = nat.rerank(*d, 0.15, 10, 100)
@@ -188,14 +200,17 @@ def hybrid_index():
 
 def test_split_hybrid_call_forms(hybrid_index):
     """The fused hybrid call (BM25 lists with -1 padding and per-query counts) through MSE_HOST, MSE_DEVICE and pinned
-    MSE_HOST_ASYNC: the split path returns what rerank_kernel returns."""
+    MSE_HOST_ASYNC: the split path returns what the two stages return with the rerank in small batches."""
     nat, bc = hybrid_index
     B = 300
     q_off, q_term, q_tf = synthetic.make_bm25_queries(bc, B, min_rank=8, seed=43, add_always=True)
     qv = synthetic.make_query_vectors(B, seed=44)
-    nat.set_option("rerank_mode", 0)
-    ref = nat.hybrid_search(q_off, q_term, q_tf, qv, 1000, 0.0, max_out=100)
-    nat.set_option("rerank_mode", 1)
+    doc, score, count = nat.bm25_search(q_off, q_term, q_tf, 1000, 0.0)
+    cand_off = np.zeros(B + 1, np.int32)
+    cand_off[1:] = np.cumsum(count)
+    cd = np.concatenate([doc[i, :count[i]] for i in range(B)]).astype(np.int32)
+    cs = np.concatenate([score[i, :count[i]] for i in range(B)]).astype(np.float32)
+    ref = _small_batch_rerank(nat, cand_off, cd, cs, qv, None, 0.15, 10, 100)
     _assert_same(nat.hybrid_search(q_off, q_term, q_tf, qv, 1000, 0.0, max_out=100), ref)
     d = tuple(torch.from_numpy(np.ascontiguousarray(a)).to(DEV) for a in (q_off, q_term, q_tf, qv))
     status = torch.zeros(4, dtype=torch.int32, device=DEV)
@@ -208,3 +223,23 @@ def test_split_hybrid_call_forms(hybrid_index):
     got = nat.hybrid_search(pin(q_off), pin(q_term), pin(q_tf), pin(qv), 1000, 0.0, max_out=100, stream=st, pinned_async=True)
     st.synchronize()
     _assert_same(got, ref)
+
+
+def test_device_query_vectors_must_be_16_byte_aligned(corpus, hybrid_index):
+    """The rerank kernels read query vectors as float4: a device pointer that is not 16-byte aligned is refused."""
+    c = corpus
+    B = 40
+    off, cd, cs = _candidates(c["n_docs"], _sizes(B, 51), 52)
+    t = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(DEV)
+    q = synthetic.make_query_vectors(B, seed=53)
+    q_bad = torch.empty(B * 768 + 1, dtype=torch.float32, device=DEV)[1:].view(B, 768)
+    q_bad.copy_(t(q))
+    with pytest.raises(_native.NativeError, match="16-byte aligned"):
+        c["nat"].rerank(t(off), t(cd), t(cs), q_bad, None, 0.15, 10, 100)
+    got = c["nat"].rerank(t(off), t(cd), t(cs), q_bad.clone(), None, 0.15, 10, 100)
+    torch.cuda.synchronize()
+    _assert_same(got, c["nat"].rerank(off, cd, cs, q, None, 0.15, 10, 100))
+    nat, bc = hybrid_index
+    q_off, q_term, q_tf = synthetic.make_bm25_queries(bc, B, min_rank=8, seed=54, add_always=True)
+    with pytest.raises(_native.NativeError, match="16-byte aligned"):
+        nat.hybrid_search(t(q_off), t(q_term), t(q_tf), q_bad, 1000, 0.0, max_out=100, n_slots=int(q_off[-1]))

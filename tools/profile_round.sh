@@ -23,6 +23,6 @@ $D256 > $OUT/plain_d256.log 2>&1 && \
 ncu --set full --clock-control none --import-source on -k regex:dense_gemm -s 2 -c 1 -o $OUT/dense_gemm_${TAG} $D256 > $OUT/ncu_d256.log 2>&1
 echo "dense_gemm rc=$?"
 H="python bench.py --steps 2 --warmup 3 --no-cpu-baseline"
-ncu --set full --clock-control none -k regex:rerank_kernel -s 2 -c 1 -o $OUT/rerank_${TAG} $H > $OUT/ncu_rerank.log 2>&1
+ncu --set full --clock-control none -k regex:rerank_gather_kernel -s 2 -c 1 -o $OUT/rerank_${TAG} $H > $OUT/ncu_rerank.log 2>&1
 echo "rerank rc=$?"
 ls -la $OUT/*.ncu-rep

@@ -12,7 +12,7 @@ ncu --metrics gpu__time_duration.sum --clock-control none -k "$OURS" -c 200 --cs
 echo "launch list rc=$?"
 ncu --set full --clock-control none --import-source on -k regex:bm25_score -s 3 -c 1 -o $OUT/bm25_score_c5_${TAG} $BENCH > $OUT/ncu_bm25_${TAG}.log 2>&1
 echo "bm25_score rc=$?"
-ncu --set full --clock-control none --import-source on -k regex:rerank_kernel -s 3 -c 1 -o $OUT/rerank_c5_${TAG} $BENCH > $OUT/ncu_rerank_${TAG}.log 2>&1
+ncu --set full --clock-control none --import-source on -k regex:rerank_gather_kernel -s 3 -c 1 -o $OUT/rerank_c5_${TAG} $BENCH > $OUT/ncu_rerank_${TAG}.log 2>&1
 echo "rerank rc=$?"
 ncu --set full --clock-control none -k regex:"topk_select|bm25_prepare" -s 6 -c 2 -o $OUT/bm25_aux_c5_${TAG} $BENCH > $OUT/ncu_aux_${TAG}.log 2>&1
 echo "aux rc=$?"
