@@ -13,6 +13,9 @@
  *                              weighting, per-doc max, sort (reranker/reranker_api.py:27-63,273-372)
  *   mse_hybrid_search_batch <- the per-query body of the batch path: bm_25.search(top_k=1000) followed by
  *                              POST /rerank (search_api.py:252-274, single query :88-102), both stages on the device
+ *   mse_diversify_batch     <- hybrid_diversification (reranker_api.py:196-236) of fused lists the caller holds
+ *   mse_hybrid_search_diversified <- the same batch path with the reranker's final diversification step (on by
+ *                              default, reranker/config.yaml:29), all three stages on the device
  *   mse_dense_scan_batch    <- the removed Retriever.quick_search (call sites search_api.py:60,87)
  *   mse_topk_merge          <- (new) merge of per-shard top-k lists after an NCCL all-gather
  *   mse_comm_* / *_sharded  <- (new) the same calls over a corpus sharded by document range across the GPUs of
@@ -48,7 +51,8 @@
  *       happen unless a large share of a corpus ties at the k-th score.
  *   [2] sharded calls: 1 when a shard list cut to m entries could hide a result of the exact top-k —
  *       repeat the call with `shard_list_len` = top_k (always exact)
- *   [3] reserved
+ *   [3] diversifying calls: number of queries whose diversified list was cut to max_out (the reference's list can be
+ *       longer than its top_k, see mse_diversify_batch)
  */
 #ifndef MSE_B200_H
 #define MSE_B200_H
@@ -82,6 +86,8 @@ extern "C" {
 
 #define MSE_STATUS_WORDS 4
 #define MSE_ST_BAD_CSR 1       /* q_off not monotone / not ending at n_slots, or a query with more than MSE_MAX_QUERY_TERMS terms */
+#define MSE_ST_BAD_LIST 2      /* diversify: an input list that is not non-increasing, in_count outside [0, in_stride] or a doc
+                                  outside the domain table */
 
 typedef struct mse_index mse_index;
 
@@ -186,7 +192,7 @@ int mse_bm25_last_stats(mse_index* idx, int64_t stats[8]);
 /* Timing hooks: every call brackets its kernels with CUDA events on the launching stream (not while the stream is
  * being captured).  Returns the accumulated device time (ms) and the number of launches since the last
  * "reset_timers"; waits for the launches still in flight.  kernel: 0 = bm25 score, 1 = top-k select,
- * 2 = dense scan, 3 = rerank, 4 = bm25 prepare, 5 = shard exchange (collectives + merges). */
+ * 2 = dense scan, 3 = rerank, 4 = bm25 prepare, 5 = shard exchange (collectives + merges), 6 = diversify. */
 int mse_kernel_time(mse_index* idx, int kernel, double* total_ms, int64_t* launches);
 
 /* ---- dense (Stage 2) ------------------------------------------------------------------- */
@@ -202,6 +208,11 @@ int mse_dense_load(mse_index* idx, int64_t n_chunks, int64_t n_docs, int64_t doc
  * reranker_api.py:44-47) in the index; the rerank / hybrid calls use it when their url_group argument is NULL.
  * n == 0 clears it. */
 int mse_dense_set_url_groups(mse_index* idx, const int32_t* url_group, int64_t n, int where);
+
+/* Stores the domain id (urlparse(url).netloc.lower(), reranker_api.py:170-176, mapped to int32 by the caller; a missing
+ * URL counts as "") of every document of the WHOLE corpus (GLOBAL dense index, n entries) in the index; the diversifying
+ * calls use it.  n == 0 clears it.  With a dense shard loaded, n must cover it: n >= doc_base + n_docs. */
+int mse_dense_set_domains(mse_index* idx, const int32_t* domain, int64_t n, int where);
 
 /* Exhaustive scan: inner product of each query with every stored chunk, max over the chunks of
  * a document, top_k documents per query (ties -> lower doc).  q is float32 [n_queries*768].
@@ -238,6 +249,37 @@ int mse_hybrid_search_batch(mse_index* idx, int32_t n_queries, int32_t n_slots, 
                             int32_t top_k, float min_score, float smoothing, int32_t max_chunks, int32_t max_out,
                             int32_t* out_doc, float* out_score, float* out_orig, int64_t* out_chunk,
                             int32_t* out_count, int32_t* out_rows, int32_t* status, int where, void* stream);
+
+/* Domain diversification (reranker_api.py:196-236) of n_queries fused lists, each sorted by score descending (ties in
+ * any order: the rule is applied to the list as given).
+ *   in_count[n_queries], in_doc / in_score / in_orig / in_chunk [n_queries * in_stride]: lists shaped like the outputs
+ *       of mse_rerank_batch (in_stride <= MSE_MAX_RERANK_CAND); in_doc is a GLOBAL dense doc index
+ *   domain       int32 per GLOBAL dense doc index, covering the documents of this index (doc_base + n_docs entries),
+ *                or NULL = the table stored by mse_dense_set_domains
+ *   relevance_threshold   a domain is hot if one of its documents has score >= it (compared in double; 0.8 in the reference)
+ *   top_k        the reference's top_k (100).  Kept documents keep their score; back-filled ones get
+ *                float(max(0, s - delta)).  The list can be longer than top_k (a reference quirk: more than top_k hot
+ *                domains); it is cut to max_out and status[3] counts the cut lists.  1 <= top_k <= max_out <= 1024.
+ *   out_*        [n_queries * max_out] (-1 / 0 padded), out_count[n_queries]; out_orig and out_chunk carry the inputs'.
+ * A bad list sets MSE_ST_BAD_LIST in status[0] and returns no result.
+ * MSE_HOST, MSE_DEVICE (enqueue-only, graph-capturable) or MSE_HOST_ASYNC. */
+int mse_diversify_batch(mse_index* idx, int32_t n_queries, int32_t in_stride, const int32_t* in_count, const int32_t* in_doc,
+                        const float* in_score, const float* in_orig, const int64_t* in_chunk, const int32_t* domain,
+                        double relevance_threshold, int32_t top_k, int32_t max_out,
+                        int32_t* out_doc, float* out_score, float* out_orig, int64_t* out_chunk, int32_t* out_count,
+                        int32_t* status, int where, void* stream);
+
+/* mse_hybrid_search_batch followed on the device by mse_diversify_batch(top_k = div_top_k) with the stored domain table:
+ * the rerank stage keeps the whole fused list of every query (up to MSE_MAX_RERANK_CAND documents), which the
+ * diversification needs (it back-fills from far down the list), and only the max_out diversified results are written.
+ * Arguments, outputs and `status` as mse_hybrid_search_batch, plus status[0] / [3] as mse_diversify_batch.
+ * MSE_ERR_STATE without a domain table covering the index. */
+int mse_hybrid_search_diversified(mse_index* idx, int32_t n_queries, int32_t n_slots, const int32_t* q_off,
+                                  const int32_t* q_term, const int32_t* q_tf, const float* q_vec,
+                                  int32_t top_k, float min_score, float smoothing, int32_t max_chunks, int32_t max_out,
+                                  int32_t* out_doc, float* out_score, float* out_orig, int64_t* out_chunk,
+                                  int32_t* out_count, int32_t* out_rows, int32_t* status, int where, void* stream,
+                                  double relevance_threshold, int32_t div_top_k);
 
 /* Sharded form of mse_rerank_batch, host-driven variant (chunk table sharded by doc range over several GPUs);
  * device buffers only (q 16-byte aligned).  Step 1, every rank: same replicated candidates; dedupes, then fills the cosines of the
@@ -301,6 +343,8 @@ int mse_hybrid_search_sharded(mse_index* idx, int32_t n_queries, int32_t n_slots
                               float smoothing, int32_t max_chunks, int32_t max_out,
                               int32_t* out_doc, float* out_score, float* out_orig, int64_t* out_chunk,
                               int32_t* out_count, int32_t* out_rows, int32_t* status, void* stream);
+/* Diversified results: call it with max_out = MSE_MAX_RERANK_CAND (the whole fused list) and pass its outputs to
+ * mse_diversify_batch on the same rank (domain table: the GLOBAL ids, mse_dense_set_domains). */
 
 /* Exhaustive dense scan over the sharded chunk table: local top_k per query, NCCL all-gather of the lists,
  * merge on every rank (replicated result: out_* are [n_queries * top_k] on every rank). */

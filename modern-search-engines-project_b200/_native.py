@@ -24,7 +24,8 @@ STATUS_WORDS = 4
 COMM_ID_BYTES = 128
 MAX_TOPK = 4096
 EMB_DIM = 768
-KERNELS = {"bm25_score": 0, "topk_select": 1, "dense_scan": 2, "rerank": 3, "bm25_prepare": 4, "exchange": 5}
+KERNELS = {"bm25_score": 0, "topk_select": 1, "dense_scan": 2, "rerank": 3, "bm25_prepare": 4, "exchange": 5,
+           "diversify": 6}
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC"]
@@ -75,9 +76,14 @@ _SIGNATURES = {
     "mse_dense_load": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int64, C.c_int64, _vp, C.c_int, _vp, C.c_int]),
     "mse_dense_scan_batch": (C.c_int, [_vp, C.c_int32, _vp, C.c_int32, _vp, _vp, _vp, C.c_int, _vp]),
     "mse_dense_set_url_groups": (C.c_int, [_vp, _vp, C.c_int64, C.c_int]),
+    "mse_dense_set_domains": (C.c_int, [_vp, _vp, C.c_int64, C.c_int]),
+    "mse_diversify_batch": (C.c_int, [_vp, C.c_int32, C.c_int32, _vp, _vp, _vp, _vp, _vp, _vp, C.c_double, C.c_int32, C.c_int32,
+                                      _vp, _vp, _vp, _vp, _vp, _vp, C.c_int, _vp]),
     "mse_dense_scan_batch_async": (C.c_int, [_vp, C.c_int32, _vp, C.c_int32, _vp, _vp, _vp, _vp, C.c_int, _vp]),
     "mse_hybrid_search_batch": (C.c_int, [_vp, C.c_int32, C.c_int32, _vp, _vp, _vp, _vp, C.c_int32, C.c_float, C.c_float, C.c_int32, C.c_int32,
                                           _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int, _vp]),
+    "mse_hybrid_search_diversified": (C.c_int, [_vp, C.c_int32, C.c_int32, _vp, _vp, _vp, _vp, C.c_int32, C.c_float, C.c_float, C.c_int32,
+                                                C.c_int32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int, _vp, C.c_double, C.c_int32]),
     "mse_comm_unique_id": (C.c_int, [_vp]),
     "mse_comm_init": (C.c_int, [_vp, _vp, C.c_int32, C.c_int32]),
     "mse_comm_attach": (C.c_int, [_vp, _vp, C.c_int32, C.c_int32]),
@@ -392,6 +398,35 @@ class NativeIndex:
         where = _where_of(url_group)
         _check(lib().mse_dense_set_url_groups(self._h, _ptr(url_group, np.int32, where), int(url_group.shape[0]), where))
 
+    def set_domains(self, domain):
+        """Stores the GLOBAL domain ids (int32 per doc, ``reranker.domain_ids``) in the index; the diversifying calls use
+        them.  None clears them."""
+        if domain is None:
+            _check(lib().mse_dense_set_domains(self._h, None, 0, MSE_HOST))
+            return
+        where = _where_of(domain)
+        _check(lib().mse_dense_set_domains(self._h, _ptr(domain, np.int32, where), int(domain.shape[0]), where))
+
+    def diversify(self, in_count, in_doc, in_score, in_orig, in_chunk, top_k: int = 100, max_out: Optional[int] = None,
+                  relevance_threshold: float = 0.8, domain=None, out=None, status=None, stream=None, pinned_async: bool = False):
+        """Domain diversification of [B, stride] fused lists (``mse_diversify_batch``); returns (doc, score, orig, chunk,
+        count) of [B, max_out] (max_out defaults to top_k).  numpy / pageable torch: MSE_HOST; CUDA tensors: MSE_DEVICE
+        (enqueue-only); pinned host tensors with ``pinned_async=True``: MSE_HOST_ASYNC.  ``domain`` None = the stored table."""
+        where = _where_of(in_count, in_doc, in_score, in_orig, in_chunk, domain)
+        if where == MSE_HOST and pinned_async:
+            where = MSE_HOST_ASYNC
+        B, stride = int(in_doc.shape[0]), int(in_doc.shape[1])
+        max_out = int(top_k if max_out is None else max_out)
+        if out is None:
+            out = self._rerank_out(B, max_out, in_doc if _is_torch(in_doc) else None, pinned=where == MSE_HOST_ASYNC)[:5]
+        _check(lib().mse_diversify_batch(self._h, B, stride, _ptr(in_count, np.int32, where), _ptr(in_doc, np.int32, where),
+                                         _ptr(in_score, np.float32, where), _ptr(in_orig, np.float32, where),
+                                         _ptr(in_chunk, np.int64, where), _ptr(domain, np.int32, where), float(relevance_threshold),
+                                         int(top_k), max_out, _ptr(out[0], np.int32, where), _ptr(out[1], np.float32, where),
+                                         _ptr(out[2], np.float32, where), _ptr(out[3], np.int64, where), _ptr(out[4], np.int32, where),
+                                         _ptr(status, np.int32, where), where, _stream_ptr(where, stream)))
+        return out
+
     @staticmethod
     def _rerank_out(B, max_out, like=None, pinned=False):
         if like is not None and _is_torch(like):
@@ -427,6 +462,28 @@ class NativeIndex:
                                              _ptr(out[0], np.int32, where), _ptr(out[1], np.float32, where), _ptr(out[2], np.float32, where),
                                              _ptr(out[3], np.int64, where), _ptr(out[4], np.int32, where), _ptr(out[5], np.int32, where),
                                              _ptr(status, np.int32, where), where, _stream_ptr(where, stream)))
+        return out
+
+    def hybrid_search_diversified(self, q_off, q_term, q_tf, q_vec, top_k: int = 1000, min_score: float = 0.0, smoothing=0.15,
+                                  max_chunks=10, max_out=100, div_top_k: int = 100, relevance_threshold: float = 0.8,
+                                  n_slots: Optional[int] = None, out=None, status=None, stream=None, pinned_async: bool = False):
+        """``hybrid_search`` followed on the device by the reranker's domain diversification (``mse_hybrid_search_diversified``,
+        needs ``set_domains``).  Buffers, ``where`` and outputs as ``hybrid_search``."""
+        where = _where_of(q_off, q_term, q_tf, q_vec)
+        if where == MSE_HOST and pinned_async:
+            where = MSE_HOST_ASYNC
+        B = int(q_off.shape[0]) - 1
+        if n_slots is None:
+            assert where != MSE_DEVICE, "pass n_slots with device-resident queries (no read-back in an enqueue-only call)"
+            n_slots = int(q_off[-1])
+        if out is None:
+            out = self._rerank_out(B, max_out, q_off if _is_torch(q_off) else None, pinned=where == MSE_HOST_ASYNC)
+        _check(lib().mse_hybrid_search_diversified(
+            self._h, B, int(n_slots), _ptr(q_off, np.int32, where), _ptr(q_term, np.int32, where), _ptr(q_tf, np.int32, where),
+            _ptr(q_vec, np.float32, where), int(top_k), float(min_score), float(smoothing), int(max_chunks), int(max_out),
+            _ptr(out[0], np.int32, where), _ptr(out[1], np.float32, where), _ptr(out[2], np.float32, where),
+            _ptr(out[3], np.int64, where), _ptr(out[4], np.int32, where), _ptr(out[5], np.int32, where),
+            _ptr(status, np.int32, where), where, _stream_ptr(where, stream), float(relevance_threshold), int(div_top_k)))
         return out
 
     # ---- corpus sharded by doc range over the GPUs of one box (NCCL inside the library) -------------------------------

@@ -16,6 +16,7 @@
 #include "comm.cuh"
 #include "common.cuh"
 #include "dense.cuh"
+#include "diversify.cuh"
 #include "gemm.cuh"
 #include "hybrid_shard.cuh"
 #include "rerank.cuh"
@@ -53,8 +54,8 @@ struct mse_index {
 
     bool has_dense = false;
     DenseDev dn{};
-    DevBuf emb, doc_chunk_off, row_doc, row_sq, tile_row, group_row, url_group;
-    int64_t n_url_groups = 0;
+    DevBuf emb, doc_chunk_off, row_doc, row_sq, tile_row, group_row, url_group, domain;
+    int64_t n_url_groups = 0, n_domains = 0;
     bool gemm_ok = false;
     int64_t n_groups = 0;
     CUtensorMap map_e;
@@ -492,6 +493,31 @@ int rerank_copy_out(const RerankArgs& a, int32_t B, int32_t max_out, int32_t* ou
     if ((rc = copy_out(out_rows, a.out_rows, sizeof(int32_t) * B, st))) return rc;
     return MSE_OK;
 }
+
+// ---- diversification core (enqueue-only) ---------------------------------------------------------------------------
+int diversify_enqueue(Lease& L, int32_t B, const DiversifyArgs& a) {
+    int t = L.timer_begin(T_DIVERSIFY);
+    diversify_kernel<<<B, kRerankThreads, 0, L.st>>>(a);
+    MSE_CUDA_TRY(cudaGetLastError());
+    L.timer_end(t);
+    return MSE_OK;
+}
+
+// the list arguments every diversifying call checks
+int diversify_checks(double threshold, int32_t top_k, int32_t max_out) {
+    MSE_REQUIRE(threshold == threshold, "relevance_threshold is NaN");
+    if (top_k < 1 || top_k > max_out || max_out > kRerankMaxCand) {
+        set_error("need 1 <= top_k (%d) <= max_out (%d) <= %d", top_k, max_out, kRerankMaxCand);
+        return MSE_ERR_UNSUPPORTED;
+    }
+    return MSE_OK;
+}
+
+// Diversification of a hybrid call (null: plain hybrid search)
+struct HybridDiversify {
+    double threshold;
+    int32_t top_k;
+};
 
 }  // namespace
 
@@ -1100,6 +1126,25 @@ int mse_dense_set_url_groups(mse_index* ix, const int32_t* url_group, int64_t n,
     return MSE_OK;
 }
 
+int mse_dense_set_domains(mse_index* ix, const int32_t* domain, int64_t n, int where) {
+    if (!ix) { set_error("null index"); return MSE_ERR_INVALID; }
+    MSE_REQUIRE(where == MSE_HOST || where == MSE_DEVICE, "bad `where`");
+    MSE_REQUIRE(n >= 0 && (n == 0 || domain), "null/negative argument");
+    std::lock_guard<std::mutex> lk(ix->mu);
+    MSE_REQUIRE(n == 0 || !ix->has_dense || n >= int64_t(ix->dn.doc_base) + ix->dn.n_docs,
+                "the domain table (%lld entries) must cover doc_base + n_docs = %lld documents", (long long)n,
+                (long long)(int64_t(ix->dn.doc_base) + ix->dn.n_docs));
+    DeviceGuard g(ix->device);
+    MSE_CUDA_TRY(cudaDeviceSynchronize());
+    ix->n_domains = 0;
+    if (n == 0) { ix->domain.release(); return MSE_OK; }
+    int rc;
+    if ((rc = ix->domain.ensure(sizeof(int32_t) * size_t(n)))) return rc;
+    MSE_CUDA_TRY(cudaMemcpy(ix->domain.p, domain, sizeof(int32_t) * size_t(n), where == MSE_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice));
+    ix->n_domains = n;
+    return MSE_OK;
+}
+
 namespace {
 // one pass of the scan + selection over queries [g0, g0 + gn) (enqueue-only)
 int dense_scan_pass(mse_index* ix, Lease& L, const float* d_q, int g0, int gn, int64_t rcap, int rtau, int32_t top_k,
@@ -1352,10 +1397,13 @@ int mse_rerank_batch(mse_index* ix, int32_t B, const int32_t* cand_off, const in
     return MSE_OK;
 }
 
-int mse_hybrid_search_batch(mse_index* ix, int32_t B, int32_t S, const int32_t* q_off, const int32_t* q_term, const int32_t* q_tf,
-                            const float* q_vec, int32_t top_k, float min_score, float smoothing, int32_t max_chunks, int32_t max_out,
-                            int32_t* out_doc, float* out_score, float* out_orig, int64_t* out_chunk, int32_t* out_count,
-                            int32_t* out_rows, int32_t* status, int where, void* stream) {
+namespace {
+// The body of mse_hybrid_search_batch and mse_hybrid_search_diversified.  With `div`, the rerank stage writes the whole
+// fused list of every query (kRerankMaxCand entries) into the workspace and diversify_kernel writes the max_out outputs.
+int hybrid_core(mse_index* ix, int32_t B, int32_t S, const int32_t* q_off, const int32_t* q_term, const int32_t* q_tf,
+                const float* q_vec, int32_t top_k, float min_score, float smoothing, int32_t max_chunks, int32_t max_out,
+                int32_t* out_doc, float* out_score, float* out_orig, int64_t* out_chunk, int32_t* out_count,
+                int32_t* out_rows, int32_t* status, int where, void* stream, const HybridDiversify* div) {
     if (!ix) { set_error("null index"); return MSE_ERR_INVALID; }
     MSE_REQUIRE(where == MSE_HOST || where == MSE_DEVICE || where == MSE_HOST_ASYNC, "bad `where`");
     MSE_REQUIRE(B >= 0 && S >= 0 && q_off && out_count && out_rows && (S == 0 || (q_term && q_tf)), "null/negative argument");
@@ -1366,13 +1414,19 @@ int mse_hybrid_search_batch(mse_index* ix, int32_t B, int32_t S, const int32_t* 
     if (max_out < 1 || max_out > kRerankMaxCand) { set_error("max_out %d outside [1, %d]", max_out, kRerankMaxCand); return MSE_ERR_UNSUPPORTED; }
     MSE_REQUIRE(smoothing >= 0.f && smoothing <= 1.f, "smoothing outside [0,1]");
     MSE_REQUIRE(min_score == min_score, "min_score is NaN");
+    int rc;
+    if (div && (rc = diversify_checks(div->threshold, div->top_k, max_out))) return rc;
     if (!ix->has_bm25) { set_error("mse_bm25_load has not been called"); return MSE_ERR_STATE; }
     if (!ix->has_dense) { set_error("mse_dense_load has not been called"); return MSE_ERR_STATE; }
     MSE_REQUIRE(ix->bm.doc_base == ix->dn.doc_base, "the BM25 and dense halves of the index must cover the same doc range");
+    const int64_t n_index_docs = int64_t(ix->dn.doc_base) + ix->dn.n_docs;
+    if (div && ix->n_domains < n_index_docs) {
+        set_error("no domain table covering the %lld documents of the index (mse_dense_set_domains)", (long long)n_index_docs);
+        return MSE_ERR_STATE;
+    }
     if (B == 0) return MSE_OK;
     DeviceGuard g(ix->device);
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    int rc;
     std::vector<int32_t> h_off;
     if (where == MSE_HOST) {
         int32_t S2 = 0;
@@ -1404,11 +1458,33 @@ int mse_hybrid_search_batch(mse_index* ix, int32_t B, int32_t S, const int32_t* 
         a.out_doc = out_doc; a.out_score = out_score; a.out_orig = out_orig; a.out_chunk = out_chunk;
         a.out_count = out_count; a.out_rows = out_rows;
     }
+    // stage 2: the rerank writes `a`'s outputs, or with `div` full lists that diversify_kernel turns into them
+    RerankArgs ra = a;
+    DiversifyArgs da{};
+    if (div) {
+        const size_t slots = size_t(B) * kRerankMaxCand;
+        if ((rc = ws->d_list[0].ensure(sizeof(int32_t) * slots))) return rc;
+        if ((rc = ws->d_list[1].ensure(sizeof(float) * slots))) return rc;
+        if ((rc = ws->d_list[2].ensure(sizeof(float) * slots))) return rc;
+        if ((rc = ws->d_list[3].ensure(sizeof(int64_t) * slots))) return rc;
+        if ((rc = ws->d_list[4].ensure(sizeof(int32_t) * size_t(B)))) return rc;
+        ra.max_out = kRerankMaxCand;
+        ra.out_doc = ws->d_list[0].as<int32_t>(); ra.out_score = ws->d_list[1].as<float>(); ra.out_orig = ws->d_list[2].as<float>();
+        ra.out_chunk = ws->d_list[3].as<int64_t>(); ra.out_count = ws->d_list[4].as<int32_t>();
+        da = DiversifyArgs{kRerankMaxCand, ra.out_count, ra.out_doc, ra.out_score, ra.out_orig, ra.out_chunk,
+                           ix->domain.as<int32_t>(), ix->n_domains, div->threshold, div->top_k, max_out,
+                           a.out_doc, a.out_score, a.out_orig, a.out_chunk, a.out_count, d_status};
+    }
+    auto stage2 = [&]() -> int {
+        int r = rerank_enqueue(ix, L, B, ra);
+        if (!r && div) r = diversify_enqueue(L, B, da);
+        return r;
+    };
     if ((rc = bm25_enqueue(ix, L, B, d_off, d_term, d_tf, S, top_k, min_score, bm25_default_cap(ix, B, top_k), ix->opt_use_tau ? 1 : 0,
                            ws->o_doc.as<int32_t>(), ws->o_score.as<float>(), ws->o_count.as<int32_t>(), nullptr, true))) return rc;
     status_add_counter_kernel<<<1, 32, 0, st>>>(reinterpret_cast<const unsigned long long*>(ws->misc.as<char>() + 40), d_status + 1);
     MSE_CUDA_TRY(cudaGetLastError());
-    if ((rc = rerank_enqueue(ix, L, B, a))) return rc;
+    if ((rc = stage2())) return rc;
     if (where == MSE_DEVICE) return MSE_OK;
     if ((rc = rerank_copy_out(a, B, max_out, out_doc, out_score, out_orig, out_chunk, out_count, out_rows, st))) return rc;
     if (where == MSE_HOST_ASYNC) {
@@ -1422,12 +1498,101 @@ int mse_hybrid_search_batch(mse_index* ix, int32_t B, int32_t S, const int32_t* 
     if (h_st[1] > 0) {
         if ((rc = bm25_search_exact(ix, L, B, S, h_off, d_off, d_term, d_tf, top_k, min_score, ws->o_doc.as<int32_t>(),
                                     ws->o_score.as<float>(), ws->o_count.as<int32_t>()))) return rc;
-        if ((rc = rerank_enqueue(ix, L, B, a))) return rc;
+        if (div) MSE_CUDA_TRY(cudaMemsetAsync(d_status + 3, 0, sizeof(int32_t), st));    // the re-run counts the cut lists again
+        if ((rc = stage2())) return rc;
         if ((rc = rerank_copy_out(a, B, max_out, out_doc, out_score, out_orig, out_chunk, out_count, out_rows, st))) return rc;
+        if (div && (rc = copy_out(&h_st[3], d_status + 3, sizeof(int32_t), st))) return rc;
         MSE_CUDA_TRY(cudaStreamSynchronize(st));
         h_st[1] = 0;
     }
     if (status) memcpy(status, h_st, sizeof(h_st));
+    return MSE_OK;
+}
+}  // namespace
+
+int mse_hybrid_search_batch(mse_index* ix, int32_t B, int32_t S, const int32_t* q_off, const int32_t* q_term, const int32_t* q_tf,
+                            const float* q_vec, int32_t top_k, float min_score, float smoothing, int32_t max_chunks, int32_t max_out,
+                            int32_t* out_doc, float* out_score, float* out_orig, int64_t* out_chunk, int32_t* out_count,
+                            int32_t* out_rows, int32_t* status, int where, void* stream) {
+    return hybrid_core(ix, B, S, q_off, q_term, q_tf, q_vec, top_k, min_score, smoothing, max_chunks, max_out, out_doc, out_score,
+                       out_orig, out_chunk, out_count, out_rows, status, where, stream, nullptr);
+}
+
+int mse_hybrid_search_diversified(mse_index* ix, int32_t B, int32_t S, const int32_t* q_off, const int32_t* q_term, const int32_t* q_tf,
+                                  const float* q_vec, int32_t top_k, float min_score, float smoothing, int32_t max_chunks, int32_t max_out,
+                                  int32_t* out_doc, float* out_score, float* out_orig, int64_t* out_chunk, int32_t* out_count,
+                                  int32_t* out_rows, int32_t* status, int where, void* stream, double relevance_threshold,
+                                  int32_t div_top_k) {
+    const HybridDiversify div{relevance_threshold, div_top_k};
+    return hybrid_core(ix, B, S, q_off, q_term, q_tf, q_vec, top_k, min_score, smoothing, max_chunks, max_out, out_doc, out_score,
+                       out_orig, out_chunk, out_count, out_rows, status, where, stream, &div);
+}
+
+int mse_diversify_batch(mse_index* ix, int32_t B, int32_t in_stride, const int32_t* in_count, const int32_t* in_doc,
+                        const float* in_score, const float* in_orig, const int64_t* in_chunk, const int32_t* domain,
+                        double relevance_threshold, int32_t top_k, int32_t max_out,
+                        int32_t* out_doc, float* out_score, float* out_orig, int64_t* out_chunk, int32_t* out_count,
+                        int32_t* status, int where, void* stream) {
+    if (!ix) { set_error("null index"); return MSE_ERR_INVALID; }
+    MSE_REQUIRE(where == MSE_HOST || where == MSE_DEVICE || where == MSE_HOST_ASYNC, "bad `where`");
+    MSE_REQUIRE(B >= 0 && out_count, "null/negative argument");
+    MSE_REQUIRE(B == 0 || (in_count && in_doc && in_score && in_orig && in_chunk && out_doc && out_score && out_orig && out_chunk),
+                "null argument");
+    if (in_stride < 1 || in_stride > kRerankMaxCand) { set_error("in_stride %d outside [1, %d]", in_stride, kRerankMaxCand); return MSE_ERR_UNSUPPORTED; }
+    int rc;
+    if ((rc = diversify_checks(relevance_threshold, top_k, max_out))) return rc;
+    int64_t n_dom = ix->n_domains;
+    if (domain) {
+        if (!ix->has_dense && !ix->has_bm25) { set_error("a domain table passed per call needs a loaded index (its size)"); return MSE_ERR_STATE; }
+        n_dom = ix->has_dense ? int64_t(ix->dn.doc_base) + ix->dn.n_docs : int64_t(ix->bm.doc_base) + ix->bm.n_docs;
+    } else if (n_dom == 0) {
+        set_error("no domain table: call mse_dense_set_domains or pass one"); return MSE_ERR_STATE;
+    }
+    if (B == 0) return MSE_OK;
+    DeviceGuard g(ix->device);
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    Lease L(&ix->pool, st);
+    Workspace* ws = L.ws;
+    int32_t* d_status;
+    if ((rc = status_begin(L, status, where, &d_status))) return rc;
+    const size_t n_in = size_t(B) * in_stride, n_out = size_t(B) * max_out;
+    DiversifyArgs a{in_stride, in_count, in_doc, in_score, in_orig, in_chunk, domain ? domain : ix->domain.as<int32_t>(), n_dom,
+                    relevance_threshold, top_k, max_out, out_doc, out_score, out_orig, out_chunk, out_count, d_status};
+    if (is_host(where)) {
+        if ((rc = ws->d_in[0].ensure(sizeof(int32_t) * size_t(B)))) return rc;
+        if ((rc = ws->d_in[1].ensure(sizeof(int32_t) * n_in))) return rc;
+        if ((rc = ws->d_in[2].ensure(sizeof(float) * n_in))) return rc;
+        if ((rc = ws->d_in[3].ensure(sizeof(float) * n_in))) return rc;
+        if ((rc = ws->d_in[4].ensure(sizeof(int64_t) * n_in))) return rc;
+        if ((rc = copy_in(ws->d_in[0].p, in_count, sizeof(int32_t) * size_t(B), where, st))) return rc;
+        if ((rc = copy_in(ws->d_in[1].p, in_doc, sizeof(int32_t) * n_in, where, st))) return rc;
+        if ((rc = copy_in(ws->d_in[2].p, in_score, sizeof(float) * n_in, where, st))) return rc;
+        if ((rc = copy_in(ws->d_in[3].p, in_orig, sizeof(float) * n_in, where, st))) return rc;
+        if ((rc = copy_in(ws->d_in[4].p, in_chunk, sizeof(int64_t) * n_in, where, st))) return rc;
+        a.in_count = ws->d_in[0].as<int32_t>(); a.in_doc = ws->d_in[1].as<int32_t>(); a.in_score = ws->d_in[2].as<float>();
+        a.in_orig = ws->d_in[3].as<float>(); a.in_chunk = ws->d_in[4].as<int64_t>();
+        if (domain) {                                      // host table passed per call: staged (prefer mse_dense_set_domains)
+            if ((rc = ws->d_in[5].ensure(sizeof(int32_t) * size_t(n_dom)))) return rc;
+            if ((rc = copy_in(ws->d_in[5].p, domain, sizeof(int32_t) * size_t(n_dom), where, st))) return rc;
+            a.domain = ws->d_in[5].as<int32_t>();
+        }
+        if ((rc = ws->r_out[0].ensure(sizeof(int32_t) * n_out))) return rc;
+        if ((rc = ws->r_out[1].ensure(sizeof(float) * n_out))) return rc;
+        if ((rc = ws->r_out[2].ensure(sizeof(float) * n_out))) return rc;
+        if ((rc = ws->r_out[3].ensure(sizeof(int64_t) * n_out))) return rc;
+        if ((rc = ws->r_out[4].ensure(sizeof(int32_t) * size_t(B)))) return rc;
+        a.out_doc = ws->r_out[0].as<int32_t>(); a.out_score = ws->r_out[1].as<float>(); a.out_orig = ws->r_out[2].as<float>();
+        a.out_chunk = ws->r_out[3].as<int64_t>(); a.out_count = ws->r_out[4].as<int32_t>();
+    }
+    if ((rc = diversify_enqueue(L, B, a))) return rc;
+    if (where == MSE_DEVICE) return MSE_OK;
+    if ((rc = copy_out(out_doc, a.out_doc, sizeof(int32_t) * n_out, st))) return rc;
+    if ((rc = copy_out(out_score, a.out_score, sizeof(float) * n_out, st))) return rc;
+    if ((rc = copy_out(out_orig, a.out_orig, sizeof(float) * n_out, st))) return rc;
+    if ((rc = copy_out(out_chunk, a.out_chunk, sizeof(int64_t) * n_out, st))) return rc;
+    if ((rc = copy_out(out_count, a.out_count, sizeof(int32_t) * size_t(B), st))) return rc;
+    if (status && (rc = copy_out(status, d_status, sizeof(int32_t) * MSE_STATUS_WORDS, st))) return rc;
+    if (where == MSE_HOST) MSE_CUDA_TRY(cudaStreamSynchronize(st));
     return MSE_OK;
 }
 

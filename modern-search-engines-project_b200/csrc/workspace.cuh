@@ -50,8 +50,8 @@ struct DevBuf {
     template <class T> T* as() const { return reinterpret_cast<T*>(p); }
 };
 
-constexpr int kNumTimers = 6;
-enum { T_SCORE = 0, T_SELECT = 1, T_SCAN = 2, T_RERANK = 3, T_PREPARE = 4, T_EXCHANGE = 5 };
+constexpr int kNumTimers = 7;
+enum { T_SCORE = 0, T_SELECT = 1, T_SCAN = 2, T_RERANK = 3, T_PREPARE = 4, T_EXCHANGE = 5, T_DIVERSIFY = 6 };
 constexpr int kTimerRing = 512;                 // event pairs per workspace: samples of calls still in flight
 constexpr int kMaxWorkspaces = 8;
 
@@ -70,6 +70,8 @@ struct Workspace {
     DevBuf best, dq, overflow, qb16, log_key, log_q;
     // rerank
     DevBuf r_in[4], r_out[6], r_split[6], r_units;
+    // diversification: full rerank lists of the hybrid call / staged inputs of mse_diversify_batch
+    DevBuf d_list[5], d_in[6];
     // merge / shard exchange
     DevBuf m_in[3], x_recv, x_merge[4], x_surv, x_gath, x_cos, x_rows, x_own, x_mm, x_rtot, x_rec, x_rrecv;
 
@@ -89,8 +91,8 @@ struct Workspace {
 };
 
 struct TimerTotals {
-    double ms[kNumTimers] = {0, 0, 0, 0, 0, 0};
-    int64_t n[kNumTimers] = {0, 0, 0, 0, 0, 0};
+    double ms[kNumTimers] = {0, 0, 0, 0, 0, 0, 0};
+    int64_t n[kNumTimers] = {0, 0, 0, 0, 0, 0, 0};
 };
 
 struct WorkspacePool {

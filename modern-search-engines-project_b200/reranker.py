@@ -7,8 +7,10 @@ FastAPI app with the same route for callers that keep the hop.
 
 On the GPU (``mse_rerank_batch``): URL-group dedupe, the <=10-chunk gather, cosine, the two pool-wide
 min-max normalisations, the 0.85/0.15 fusion, positional weighting, per-doc max and the sort.
-On the host, as string/URL logic (SURVEY.md §8f N2): domain diversification (``:170-236``) and the
-response objects (``:374-412``).
+On the host, as string/URL logic (SURVEY.md §8f N2): the URL -> domain id mapping (``domain_ids``) and the response
+objects (``:374-412``).  Domain diversification (``:196-236``) runs on the host in ``rerank`` and in
+``hybrid_diversification``, and on the device (``mse_diversify_batch``) in ``rerank_batch(diversify=True)`` and
+``pipeline.HybridSearch.search_batch_device``.
 """
 from __future__ import annotations
 
@@ -117,6 +119,16 @@ def url_groups(urls: Sequence[Optional[str]]) -> np.ndarray:
     return out
 
 
+def domain_ids(urls: Sequence[Optional[str]]) -> np.ndarray:
+    """int32 id per doc of ``extract_domain(url)`` (None counts as ``""``, as both host paths pass ``url or ""``): docs
+    share an id exactly when ``hybrid_diversification`` puts them in the same domain."""
+    keys: Dict[str, int] = {}
+    out = np.empty(len(urls), dtype=np.int32)
+    for i, u in enumerate(urls):
+        out[i] = keys.setdefault(extract_domain(u or ""), len(keys))
+    return out
+
+
 class Reranker:
     def __init__(self, store, doc_ids: np.ndarray, native: Optional[_native.NativeIndex] = None, *, device: int = 0,
                  embed: Optional[Callable[[str], np.ndarray]] = None, smoothing: float = SMOOTHING, top_k: int = TOP_K,
@@ -140,14 +152,21 @@ class Reranker:
         self._urls = [url_map.get(int(d)) for d in self.doc_ids.tolist()] if url_map else None
         self.url_group = url_groups(self._urls) if self._urls is not None else None
         self._in_urls = np.asarray([u is not None for u in self._urls]) if self._urls is not None else None
+        self.domain = domain_ids(self._urls) if self._urls is not None else None
         if self.url_group is not None:                       # uploaded once; the rerank calls use the stored groups
             self.native.set_url_groups(np.ascontiguousarray(self.url_group, dtype=np.int32))
+            if hasattr(self.native, "set_domains"):          # ... and the diversifying calls the stored domains
+                self.native.set_domains(self.domain)
 
     # ---- batched numeric core ------------------------------------------------------------------------
     def rerank_batch(self, cand_idx: Sequence[np.ndarray], cand_score: Sequence[np.ndarray], q_vecs: np.ndarray,
-                     max_out: int = 1000):
+                     max_out: int = 1000, diversify: bool = False):
         """``cand_idx[i]``: dense doc indices of query i in BM25 order; returns per-query arrays
-        (doc index, fused score, min-max'd BM25 score, chunk id of the best window, count, fetched rows)."""
+        (doc index, fused score, min-max'd BM25 score, chunk id of the best window, count, fetched rows).
+        ``diversify=True``: the whole fused list of every query (up to 1024 documents) goes through the device domain
+        diversification with this reranker's ``top_k`` (``hybrid_diversification``'s result, cut to ``max_out``)."""
+        if diversify and self.domain is None:
+            raise ValueError("diversify=True needs the documents' URLs (the store has no urls())")
         off = np.zeros(len(cand_idx) + 1, dtype=np.int32)
         docs, sims = [], []
         for i, (d, s) in enumerate(zip(cand_idx, cand_score)):
@@ -161,7 +180,10 @@ class Reranker:
         q = np.ascontiguousarray(q_vecs, dtype=np.float32).reshape(len(cand_idx), _native.EMB_DIM)
         o_doc, o_score, o_orig, o_chunk, o_count, o_rows = self.native.rerank(
             off, np.ascontiguousarray(cd), np.ascontiguousarray(cs), q, None, self.smoothing,
-            self.max_chunks, max_out)
+            self.max_chunks, _native.NativeIndex.MAX_CAND if diversify else max_out)
+        if diversify:
+            o_doc, o_score, o_orig, o_chunk, o_count = self.native.diversify(
+                o_count, o_doc, o_score, o_orig, o_chunk, top_k=self.top_k, max_out=max_out)
         o_chunk = np.where(o_chunk >= 0, self.chunk_ids[np.maximum(o_chunk, 0)] if len(self.chunk_ids) else -1, -1)
         return o_doc, o_score, o_orig, o_chunk, o_count, o_rows
 
